@@ -81,11 +81,8 @@ def ps_matrix(clusters, counts, device=0):
         raise ValueError("inclusion counts must be non-negative integers below 2^31")
     listing = {n: clusters.get(n, [""]) for n in all_names}
     row_ptr, col_idx = jn.csr_from_named_lists(all_names, listing, "sum")
-    dev = torch.device("cuda", device)
-    S = dense.shape[1]
-    buf = torch.zeros((len(all_names), (S + 3) // 4 * 4), dtype=torch.int32, device=dev)
-    buf[:, :S] = torch.from_numpy(as_int.astype(np.int32)).to(dev)
-    ps = ops.quant_ps(buf[:, :S], row_ptr, col_idx, want_f32=False, want_f64=True, row_end=len(names))["ps_f64"]
+    inc = ops.upload_counts(as_int, torch.device("cuda", device))
+    ps = ops.quant_ps(inc, row_ptr, col_idx, want_f32=False, want_f64=True, row_end=len(names))["ps_f64"]
     return names, ps[:len(names)].cpu().numpy()
 
 

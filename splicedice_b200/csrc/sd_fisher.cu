@@ -9,7 +9,7 @@
 // single shared-memory copy of the double-double log-factorial table; a group takes up to 2,048
 // pairs of one junction, stages the junction's inclusion / exclusion row in shared memory,
 // counting-sorts the pairs by predicted tail length and hands out groups of 32 similar pairs to
-// its warps.  Fallback / 64-bit totals: one warp per (junction, 32-pair tile) in pair order.
+// its warps.  64-bit totals: one warp per (junction, 32-pair tile) in pair order.
 // Entries beyond the staged table prefix come from the global copy through L1/L2.  The kernel is
 // FP64-pipe / issue bound: 7 FP64 instructions per summed tail term, no division or exp in the
 // loop, cut and rescale tests on the exponent words with integer instructions.
@@ -128,12 +128,13 @@ __device__ __forceinline__ void stage_table(double2 *s_tab, const double2 *g_tab
     __syncthreads();
 }
 
-template <class Int, int kMode>
+// Pair-order kernel: tables whose totals reach 2^30 (64-bit arithmetic), which always extend
+// beyond the device table (mode 2).
 __global__ void __launch_bounds__(kFisherThreads, 3) fisher_pairwise_kernel(const FisherParams p)
 {
     extern __shared__ __align__(16) double2 s_tab[];
     stage_table(s_tab, p.table, p.smem_entries);
-    const DeviceTable<kMode> tab{smem_u32(s_tab), p.table, p.smem_entries, p.table_entries};
+    const DeviceTable<2> tab{smem_u32(s_tab), p.table, p.smem_entries, p.table_entries};
 
     const int lane = threadIdx.x & 31;
     const int64_t tiles_per_row = (p.n_pairs + 31) / 32;
@@ -155,7 +156,7 @@ __global__ void __launch_bounds__(kFisherThreads, 3) fisher_pairwise_kernel(cons
             if (a64 < 0 || b64 < 0 || c64 < 0 || d64 < 0 || a64 + c64 > p.cell_bound || b64 + d64 > p.cell_bound)
                 pv = __longlong_as_double(0x7FF8000000000000ll);
             else
-                pv = fisher::two_sided<Int>(tab, (Int)a64, (Int)b64, (Int)c64, (Int)d64);
+                pv = fisher::two_sided<int64_t>(tab, a64, b64, c64, d64);
             store_p(p, j, k, pv);
         }
         j += dj;
@@ -167,7 +168,7 @@ __global__ void __launch_bounds__(kFisherThreads, 3) fisher_pairwise_kernel(cons
 // ---- binned form: lanes of a warp get tables of similar cost -----------------------------------
 // The tail sums dominate the work and their length varies several-fold between the pairs of one
 // junction (it grows with the hypergeometric sigma and shrinks with the observed table's
-// distance from the mode), so in the plain kernel a warp waits for its longest lane: 56 % lane
+// distance from the mode), so in the pair-order kernel a warp waits for its longest lane: 56 % lane
 // occupancy in the tail loops.  Here a CTA takes up to 2,048 pairs of one junction, predicts the
 // number of tail terms of each table in binary32,
 //     terms ~ sigma * (sqrt(z^2 + 2 ln 2^48) - z),   z = |a - mode| / sigma
@@ -403,6 +404,8 @@ __global__ void __launch_bounds__(256) fisher_scan_tables(int64_t n, const int64
 // ---- device copies of the table: one per device, grown on demand, never shrunk ----------
 namespace {
 constexpr int64_t kTableCap = int64_t(1) << 22;      // 4 Mi entries = 64 MB; beyond: fisher::lgfact_stirling
+// totals that need 64-bit integers are always beyond the table: their kernels need table mode 2 only
+static_assert(kTableCap < (int64_t(1) << 30), "64-bit totals must lie beyond the device table");
 constexpr int kMaxDevices = 64;
 std::mutex g_tab_mu;
 double2 *g_tab_dev[kMaxDevices] = {};
@@ -464,23 +467,16 @@ static int fisher_grid(const void *kernel, size_t smem, int threads = kFisherThr
     return sms * per_sm;
 }
 
-// instantiation for (largest table total, table coverage)
-template <template <class, int> class Launcher, class... Args>
-static int dispatch(int64_t max_total, int64_t smem_entries, int64_t table_entries, Args... args)
+// table coverage of the largest table total: 0 inside the staged prefix, 1 inside the device
+// table, 2 beyond it (Stirling series)
+static int table_mode(int64_t max_total, int64_t smem_entries, int64_t table_entries)
 {
-    const bool small = max_total < (int64_t(1) << 30);
-    const int mode = max_total < smem_entries ? 0 : (max_total < table_entries ? 1 : 2);
-    if (small) {
-        if (mode == 0) return Launcher<int32_t, 0>::run(args...);
-        if (mode == 1) return Launcher<int32_t, 1>::run(args...);
-        return Launcher<int32_t, 2>::run(args...);
-    }
-    if (mode == 1) return Launcher<int64_t, 1>::run(args...);
-    return Launcher<int64_t, 2>::run(args...);
+    return max_total < smem_entries ? 0 : (max_total < table_entries ? 1 : 2);
 }
 
-template <class Int, int kMode>
-struct PairwiseLauncher {
+// every table total fits 31 bits: the cost-binned kernel
+template <int kMode>
+struct BinnedLauncher {
     template <int kSub, bool kStaged>
     static int launch_binned(const FisherParams &p, cudaStream_t stream)
     {
@@ -506,40 +502,51 @@ struct PairwiseLauncher {
     }
     static int run(const FisherParams &p, cudaStream_t stream)
     {
-        if (p.binned) {
-            // every table total fits 31 bits: the cost-binned kernel, 4 x 256 threads per SM when the
-            // whole table is staged (64 registers, no spills), 3 x 256 otherwise
-            constexpr int kSub = kMode == 0 ? 4 : 3;
-            return p.n_samples <= kStageSamples ? launch_binned<kSub, true>(p, stream)
-                                                : launch_binned<kSub, false>(p, stream);
-        }
-        auto kernel = fisher_pairwise_kernel<Int, kMode>;
-        const size_t smem = (size_t)p.smem_entries * sizeof(double2);
-        SD_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)(kSmemEntriesMax * sizeof(double2))));
-        const int64_t items = (p.row_end - p.row_begin) * ((p.n_pairs + 31) / 32);
-        int grid = fisher_grid((const void *)kernel, smem);
-        grid = (int)std::min<int64_t>(grid, (items + kFisherThreads / 32 - 1) / (kFisherThreads / 32));
-        kernel<<<grid, kFisherThreads, smem, stream>>>(p);
-        return check_launch("fisher_pairwise_kernel");
+        // 4 x 256 threads per SM when the whole table is staged (64 registers, no spills), 3 x 256 otherwise
+        constexpr int kSub = kMode == 0 ? 4 : 3;
+        return p.n_samples <= kStageSamples ? launch_binned<kSub, true>(p, stream)
+                                            : launch_binned<kSub, false>(p, stream);
     }
 };
 
+static int launch_pair_order(const FisherParams &p, cudaStream_t stream)
+{
+    auto kernel = fisher_pairwise_kernel;
+    const size_t smem = (size_t)p.smem_entries * sizeof(double2);
+    SD_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)(kSmemEntriesMax * sizeof(double2))));
+    const int64_t items = (p.row_end - p.row_begin) * ((p.n_pairs + 31) / 32);
+    int grid = fisher_grid((const void *)kernel, smem);
+    grid = (int)std::min<int64_t>(grid, (items + kFisherThreads / 32 - 1) / (kFisherThreads / 32));
+    kernel<<<grid, kFisherThreads, smem, stream>>>(p);
+    return check_launch("fisher_pairwise_kernel");
+}
+
 template <class Int, int kMode>
-struct TablesLauncher {
-    static int run(int64_t n, const int64_t *a, const int64_t *b, const int64_t *c, const int64_t *d, double *out,
-                   const double2 *table, int64_t entries, int32_t smem_entries, cudaStream_t stream)
-    {
-        auto kernel = fisher_tables_kernel<Int, kMode>;
-        const size_t smem = (size_t)smem_entries * sizeof(double2);
-        SD_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)(kSmemEntriesMax * sizeof(double2))));
-        int grid = fisher_grid((const void *)kernel, smem);
-        grid = (int)std::min<int64_t>(grid, (n + kFisherThreads - 1) / kFisherThreads);
-        kernel<<<grid, kFisherThreads, smem, stream>>>(n, a, b, c, d, out, table, entries, smem_entries);
-        return check_launch("fisher_tables_kernel");
+static int launch_tables(int64_t n, const int64_t *a, const int64_t *b, const int64_t *c, const int64_t *d, double *out,
+                         const double2 *table, int64_t entries, int32_t smem_entries, cudaStream_t stream)
+{
+    auto kernel = fisher_tables_kernel<Int, kMode>;
+    const size_t smem = (size_t)smem_entries * sizeof(double2);
+    SD_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)(kSmemEntriesMax * sizeof(double2))));
+    int grid = fisher_grid((const void *)kernel, smem);
+    grid = (int)std::min<int64_t>(grid, (n + kFisherThreads - 1) / kFisherThreads);
+    kernel<<<grid, kFisherThreads, smem, stream>>>(n, a, b, c, d, out, table, entries, smem_entries);
+    return check_launch("fisher_tables_kernel");
+}
+
+// instantiation of fisher_tables_kernel for (largest table total, table coverage)
+template <class... Args>
+static int dispatch(int64_t max_total, int64_t smem_entries, int64_t table_entries, Args... args)
+{
+    if (max_total >= (int64_t(1) << 30)) return launch_tables<int64_t, 2>(args...);
+    switch (table_mode(max_total, smem_entries, table_entries)) {
+    case 0: return launch_tables<int32_t, 0>(args...);
+    case 1: return launch_tables<int32_t, 1>(args...);
+    default: return launch_tables<int32_t, 2>(args...);
     }
-};
+}
 
 // max over rows [row_begin, row_end) of inc + exc (a table total is at most twice that);
 // SD_ERR_INVALID on a negative entry.  Synchronises the stream.
@@ -563,11 +570,37 @@ int launch_fisher_pairwise(FisherParams p, cudaStream_t stream, int64_t max_cell
         if (int rc = fisher_max_cell(p, stream, &max_cell)) return rc;
     const int64_t max_total = 2 * max_cell;
     p.cell_bound = max_cell;
-    p.binned = max_total < (int64_t(1) << 30) && !getenv("SD_FISHER_PLAIN");
+    p.binned = max_total < (int64_t(1) << 30);
     if (int rc = device_table(max_total + 1, &p.table, &p.table_entries, stream)) return rc;
     p.smem_entries = (int32_t)std::min<int64_t>(std::min<int64_t>(max_total + 1, p.table_entries),
                                                 p.binned ? kSmemEntriesBinned : kSmemEntriesMax);
-    return dispatch<PairwiseLauncher>(max_total, p.smem_entries, p.table_entries, p, stream);
+    if (!p.binned) return launch_pair_order(p, stream);
+    switch (table_mode(max_total, p.smem_entries, p.table_entries)) {
+    case 0: return BinnedLauncher<0>::run(p, stream);
+    case 1: return BinnedLauncher<1>::run(p, stream);
+    default: return BinnedLauncher<2>::run(p, stream);
+    }
+}
+
+// Checks and FisherParams fill shared by the device-pointer entry points (`who` names the entry point
+// in the messages); *empty: no rows or no pairs, nothing to launch.
+static int pairwise_params(const char *who, int64_t n_junctions, int32_t n_samples, const int32_t *inc,
+                           int64_t ld_inc, const int64_t *exc, int64_t ld_exc, int64_t n_pairs, const int32_t *pair_a,
+                           const int32_t *pair_b, int64_t row_begin, int64_t row_end, FisherParams *p, bool *empty)
+{
+    SD_REQUIRE(n_junctions >= 0 && n_samples >= 0 && n_pairs >= 0, "%s: negative size", who);
+    SD_REQUIRE(row_begin >= 0 && row_begin <= row_end && row_end <= n_junctions,
+               "%s: row range outside [0, n_junctions)", who);
+    *empty = row_begin == row_end || n_pairs == 0;
+    if (*empty) return SD_OK;
+    SD_REQUIRE(inc && exc && pair_a && pair_b, "%s: null pointer", who);
+    SD_REQUIRE(ld_inc >= n_samples && ld_exc >= n_samples, "%s: ld too small", who);
+    *p = FisherParams{};
+    p->n_junctions = n_junctions; p->n_samples = n_samples;
+    p->inc = inc; p->ld_inc = ld_inc; p->exc = exc; p->ld_exc = ld_exc;
+    p->n_pairs = n_pairs; p->pair_a = pair_a; p->pair_b = pair_b;
+    p->row_begin = row_begin; p->row_end = row_end;
+    return SD_OK;
 }
 
 }  // namespace sd
@@ -579,17 +612,15 @@ int sd_fisher_pairwise(int64_t n_junctions, int32_t n_samples, const int32_t *in
                        const int32_t *pair_b, double *p_out, int64_t ld_p, int64_t row_begin,
                        int64_t row_end, void *stream)
 {
-    SD_REQUIRE(n_junctions >= 0 && n_samples >= 0 && n_pairs >= 0, "sd_fisher_pairwise: negative size");
-    SD_REQUIRE(row_begin >= 0 && row_begin <= row_end && row_end <= n_junctions,
-               "sd_fisher_pairwise: row range outside [0, n_junctions)");
-    if (row_begin == row_end || n_pairs == 0) return SD_OK;
-    SD_REQUIRE(inc && exc && pair_a && pair_b && p_out, "sd_fisher_pairwise: null pointer");
-    SD_REQUIRE(ld_inc >= n_samples && ld_exc >= n_samples && ld_p >= n_pairs, "sd_fisher_pairwise: ld too small");
-    sd::FisherParams p{};
-    p.n_junctions = n_junctions; p.n_samples = n_samples;
-    p.inc = inc; p.ld_inc = ld_inc; p.exc = exc; p.ld_exc = ld_exc;
-    p.n_pairs = n_pairs; p.pair_a = pair_a; p.pair_b = pair_b;
-    p.p_out = p_out; p.ld_p = ld_p; p.row_begin = row_begin; p.row_end = row_end;
+    sd::FisherParams p;
+    bool empty;
+    if (int rc = sd::pairwise_params("sd_fisher_pairwise", n_junctions, n_samples, inc, ld_inc, exc, ld_exc, n_pairs,
+                                     pair_a, pair_b, row_begin, row_end, &p, &empty))
+        return rc;
+    if (empty) return SD_OK;
+    SD_REQUIRE(p_out, "sd_fisher_pairwise: null pointer");
+    SD_REQUIRE(ld_p >= n_pairs, "sd_fisher_pairwise: ld too small");
+    p.p_out = p_out; p.ld_p = ld_p;
     return sd::launch_fisher_pairwise(p, (cudaStream_t)stream, -1);
 }
 
@@ -598,18 +629,16 @@ int sd_fisher_pairwise_bounded(int64_t n_junctions, int32_t n_samples, const int
                                const int32_t *pair_b, double *p_out, int64_t ld_p, int64_t row_begin,
                                int64_t row_end, int64_t max_cell_bound, void *stream)
 {
-    SD_REQUIRE(n_junctions >= 0 && n_samples >= 0 && n_pairs >= 0, "sd_fisher_pairwise_bounded: negative size");
-    SD_REQUIRE(row_begin >= 0 && row_begin <= row_end && row_end <= n_junctions,
-               "sd_fisher_pairwise_bounded: row range outside [0, n_junctions)");
     SD_REQUIRE(max_cell_bound >= 0 && max_cell_bound < (int64_t(1) << 61), "sd_fisher_pairwise_bounded: bad bound");
-    if (row_begin == row_end || n_pairs == 0) return SD_OK;
-    SD_REQUIRE(inc && exc && pair_a && pair_b && p_out, "sd_fisher_pairwise_bounded: null pointer");
-    SD_REQUIRE(ld_inc >= n_samples && ld_exc >= n_samples && ld_p >= n_pairs, "sd_fisher_pairwise_bounded: ld too small");
-    sd::FisherParams p{};
-    p.n_junctions = n_junctions; p.n_samples = n_samples;
-    p.inc = inc; p.ld_inc = ld_inc; p.exc = exc; p.ld_exc = ld_exc;
-    p.n_pairs = n_pairs; p.pair_a = pair_a; p.pair_b = pair_b;
-    p.p_out = p_out; p.ld_p = ld_p; p.row_begin = row_begin; p.row_end = row_end;
+    sd::FisherParams p;
+    bool empty;
+    if (int rc = sd::pairwise_params("sd_fisher_pairwise_bounded", n_junctions, n_samples, inc, ld_inc, exc, ld_exc,
+                                     n_pairs, pair_a, pair_b, row_begin, row_end, &p, &empty))
+        return rc;
+    if (empty) return SD_OK;
+    SD_REQUIRE(p_out, "sd_fisher_pairwise_bounded: null pointer");
+    SD_REQUIRE(ld_p >= n_pairs, "sd_fisher_pairwise_bounded: ld too small");
+    p.p_out = p_out; p.ld_p = ld_p;
     return sd::launch_fisher_pairwise(p, (cudaStream_t)stream, max_cell_bound);
 }
 
@@ -619,22 +648,18 @@ int sd_fisher_pairwise_scatter(int64_t n_junctions, int32_t n_samples, const int
                                const int64_t *dest_ld, int64_t dest_row_offset, int64_t row_begin, int64_t row_end,
                                int64_t max_cell_bound, void *stream)
 {
-    SD_REQUIRE(n_junctions >= 0 && n_samples >= 0 && n_pairs >= 0, "sd_fisher_pairwise_scatter: negative size");
-    SD_REQUIRE(row_begin >= 0 && row_begin <= row_end && row_end <= n_junctions,
-               "sd_fisher_pairwise_scatter: row range outside [0, n_junctions)");
     SD_REQUIRE(max_cell_bound >= 0 && max_cell_bound < (int64_t(1) << 61), "sd_fisher_pairwise_scatter: bad bound");
     SD_REQUIRE(n_dest >= 1 && n_dest <= sd::kMaxDest, "sd_fisher_pairwise_scatter: 1..%d destinations", sd::kMaxDest);
     SD_REQUIRE(n_pairs < (int64_t(1) << 31), "sd_fisher_pairwise_scatter: too many pairs");
-    if (row_begin == row_end || n_pairs == 0) return SD_OK;
-    SD_REQUIRE(inc && exc && pair_a && pair_b && dest && dest_col_begin && dest_ld, "sd_fisher_pairwise_scatter: null pointer");
-    SD_REQUIRE(ld_inc >= n_samples && ld_exc >= n_samples, "sd_fisher_pairwise_scatter: ld too small");
+    sd::FisherParams p;
+    bool empty;
+    if (int rc = sd::pairwise_params("sd_fisher_pairwise_scatter", n_junctions, n_samples, inc, ld_inc, exc, ld_exc,
+                                     n_pairs, pair_a, pair_b, row_begin, row_end, &p, &empty))
+        return rc;
+    if (empty) return SD_OK;
+    SD_REQUIRE(dest && dest_col_begin && dest_ld, "sd_fisher_pairwise_scatter: null pointer");
     SD_REQUIRE(dest_col_begin[0] == 0 && dest_col_begin[n_dest] == n_pairs,
                "sd_fisher_pairwise_scatter: the column blocks must cover [0, n_pairs)");
-    sd::FisherParams p{};
-    p.n_junctions = n_junctions; p.n_samples = n_samples;
-    p.inc = inc; p.ld_inc = ld_inc; p.exc = exc; p.ld_exc = ld_exc;
-    p.n_pairs = n_pairs; p.pair_a = pair_a; p.pair_b = pair_b;
-    p.p_out = nullptr; p.ld_p = 0; p.row_begin = row_begin; p.row_end = row_end;
     p.n_dest = n_dest; p.dest_row0 = dest_row_offset;
     for (int g = 0; g < n_dest; ++g) {
         const int64_t width = dest_col_begin[g + 1] - dest_col_begin[g];
@@ -668,8 +693,8 @@ int sd_fisher_tables(int64_t n_tables, const int64_t *a, const int64_t *b, const
     if ((rc = sd::device_table(max_total + 1, &table, &entries, stream)) != SD_OK) return rc;
     const int32_t smem_entries =
         (int32_t)std::min<int64_t>(std::min<int64_t>(max_total + 1, entries), sd::kSmemEntriesMax);
-    return sd::dispatch<sd::TablesLauncher>(max_total, (int64_t)smem_entries, entries, n_tables, a, b, c, d, p_out, table,
-                                            entries, smem_entries, stream);
+    return sd::dispatch(max_total, (int64_t)smem_entries, entries, n_tables, a, b, c, d, p_out, table, entries,
+                        smem_entries, stream);
 }
 
 }  // extern "C"

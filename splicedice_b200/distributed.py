@@ -105,12 +105,7 @@ def quant_ps_sharded(counts_host, row_ptr, col_idx, device=None, gather=True, lo
     parts = sharding.partition_rows(row_ptr, col_idx, _world()[1], sharding.row_weights(row_ptr, n_cols))
 
     def slab(counts_slab, rp, ci):
-        c = torch.from_numpy(np.ascontiguousarray(counts_slab, dtype=np.int32)).to(dev)
-        n = c.shape[1]
-        if n % 4:                                  # 16-byte row alignment for the tiled kernels
-            buf = torch.zeros((c.shape[0], (n + 3) // 4 * 4), dtype=torch.int32, device=dev)
-            buf[:, :n] = c
-            c = buf[:, :n]
+        c = ops.upload_counts(counts_slab, dev)
         mask = None
         if low_mask is not None:
             r0, r1 = parts[rank]
@@ -320,6 +315,7 @@ def pairwise_sharded(counts_host, row_ptr, col_idx, correction="pairwise", devic
     rank's row slab, then the correction.  counts_host: integer [J, S] on every rank (each uploads
     only its slab).  Returns (float64 CUDA tensor [rows_r, P], (r0, r1))."""
     from . import ops
+    from .pairwise_fisher import checked_counts, fisher_inputs
     rank, world = _world()
     if correction not in ("none", "pairwise", "all"):
         raise ValueError("correction must be 'none', 'pairwise' or 'all'")
@@ -327,18 +323,7 @@ def pairwise_sharded(counts_host, row_ptr, col_idx, correction="pairwise", devic
     parts = sharding.partition_rows(row_ptr, col_idx, world)
     r0, r1 = parts[rank]
     rp, ci = sharding.shard_csr(row_ptr, col_idx, r0, r1)
-    slab = np.ascontiguousarray(counts_host[r0:r1]).astype(np.int64)
-    if (slab < 0).any():
-        raise ValueError("All values in `table` must be nonnegative.")
-    if (slab >= 2 ** 31).any():                     # the same guard pairwise_fisher.pairwise_pvalues has
-        raise ValueError("counts of 2^31 and above are not supported")
-    S = slab.shape[1]
-    buf = torch.zeros((r1 - r0, (S + 3) // 4 * 4), dtype=torch.int32, device=dev)
-    buf[:, :S] = torch.from_numpy(slab.astype(np.int32)).to(dev)
-    inc = buf[:, :S]
-    exc = ops.quant_ps(inc, rp, ci, want_f32=False, want_exc=True)["exc"]
-    pa, pb = ops.all_pairs(S)
-    bound = int(slab.max(initial=0)) * (1 + int(np.diff(rp).max(initial=0)))
+    inc, exc, pa, pb, bound = fisher_inputs(checked_counts(counts_host[r0:r1]), rp, ci, dev)
     if correction == "pairwise" and 1 < world <= FUSED_MAX_WORLD and dist.get_backend() == "nccl" and len(pa) >= world:
         # the exchange rides on the kernels' own stores (peer memory); see pairwise_fused
         return pairwise_fused(inc, exc, pa, pb, parts, bound).clone(), (r0, r1)

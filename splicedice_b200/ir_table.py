@@ -166,12 +166,11 @@ def calculateIR(samples, coverageDirectory, counts, clusters, annotated, args, d
     if (inc < 0).any() or (inc >= 2 ** 31).any():
         raise ValueError("inclusion counts must be non-negative integers below 2^31")
     dev = torch.device("cuda", device)
-    buf = torch.zeros((len(all_names), (S + 3) // 4 * 4), dtype=torch.int32, device=dev)
-    buf[:, :S] = torch.from_numpy(inc.astype(np.int32)).to(dev)
+    inc_d = ops.upload_counts(inc, dev)
     med = torch.zeros((len(all_names), S), dtype=torch.float64, device=dev)
     med[:J] = torch.from_numpy(median).to(dev)
     if clusters is None or args.singleJunctionCalculation:
-        ir = ops.ir_ratio(med, buf[:, :S], row_end=J)
+        ir = ops.ir_ratio(med, inc_d, row_end=J)
     else:
         row_ptr = np.zeros(len(all_names) + 1, dtype=np.int64)
         cols = []
@@ -179,7 +178,7 @@ def calculateIR(samples, coverageDirectory, counts, clusters, annotated, args, d
             cols.extend(all_index[o] for o in clusters[n])
             row_ptr[r + 1] = len(cols)
         row_ptr[J + 1:] = len(cols)
-        ir = ops.ir_ratio(med, buf[:, :S], row_ptr.astype(np.int32), np.asarray(cols, dtype=np.int32), row_end=J)
+        ir = ops.ir_ratio(med, inc_d, row_ptr.astype(np.int32), np.asarray(cols, dtype=np.int32), row_end=J)
     ir = ir[:J].cpu().numpy()
     rsd = ops.rsd5(torch.from_numpy(cov).to(dev)).cpu().numpy()
     keep = np.flatnonzero((rsd < args.RSDthreshold).any(axis=1))

@@ -89,6 +89,15 @@ def cluster_build(chrom_rank, strand_rank, start, end, device=None, with_adjacen
 # ---------------------------------------------------------------------------------------
 # K2
 # ---------------------------------------------------------------------------------------
+def upload_counts(host_matrix, device):
+    """int32 CUDA view [J, S] of a host integer matrix (values already checked to fit int32), in a
+    zero-padded [J, ceil4(S)] buffer: the tiled count kernels need 16-byte aligned rows."""
+    J, S = host_matrix.shape
+    buf = torch.zeros((J, (S + 3) // 4 * 4), dtype=torch.int32, device=device)
+    buf[:, :S] = torch.from_numpy(np.ascontiguousarray(host_matrix, dtype=np.int32)).to(device)
+    return buf[:, :S]
+
+
 def quant_ps(counts, row_ptr, col_idx, low_mask=None, want_f32=True, want_f64=False, want_exc=False,
              row_begin=0, row_end=None, flags=native.SD_QUANT_AUTO, out_f32=None, out_f64=None, out_exc=None):
     """PS (float32 as SPLICEDICE.calculatePsi, float64 as counts_to_ps) and/or exclusion sums
@@ -179,36 +188,6 @@ def fisher_pairwise(inc, exc, pair_a, pair_b, row_begin=0, row_end=None, out=Non
                         exc.stride(0), P, native.ptr(pa), native.ptr(pb), native.ptr(out), out.stride(0), row_begin,
                         row_end, int(max_cell_bound), _sp())
     return out
-
-
-def fisher_pairwise_scatter(inc, exc, pair_a, pair_b, dests, col_begin, dest_row_offset, max_cell_bound,
-                            row_begin=0, row_end=None):
-    """sd_fisher_pairwise_scatter: the p-value of (row j, pair k) is stored into ``dests[g][dest_row_offset + j,
-    k - col_begin[g]]`` for the block g that owns column k.  ``dests``: float64 CUDA matrices (possibly
-    peer-GPU memory); ``col_begin``: the n_dest + 1 column cuts."""
-    require_cuda()
-    if inc.dtype != torch.int32 or exc.dtype != torch.int64 or not inc.is_cuda or not exc.is_cuda:
-        raise TypeError("fisher_pairwise_scatter: inc int32 / exc int64 CUDA tensors expected")
-    J, S = inc.shape
-    dev = inc.device
-    pa, pb = _i32(pair_a, dev), _i32(pair_b, dev)
-    P = int(pa.numel())
-    n = len(dests)
-    if len(col_begin) != n + 1 or col_begin[0] != 0 or col_begin[-1] != P:
-        raise ValueError("fisher_pairwise_scatter: col_begin must hold n_dest + 1 cuts covering all pairs")
-    for g, t in enumerate(dests):
-        if t.dtype != torch.float64 or not t.is_cuda or t.dim() != 2 or (t.numel() and t.stride(1) != 1):
-            raise TypeError("fisher_pairwise_scatter: destinations must be 2-D float64 CUDA tensors with unit column stride")
-        if t.shape[1] < col_begin[g + 1] - col_begin[g] or t.shape[0] < dest_row_offset + (J if row_end is None else row_end):
-            raise ValueError(f"fisher_pairwise_scatter: destination {g} is too small")
-    ptrs = (ctypes.c_void_p * n)(*[t.data_ptr() for t in dests])
-    cols = (ctypes.c_int64 * (n + 1))(*[int(c) for c in col_begin])
-    lds = (ctypes.c_int64 * n)(*[int(t.stride(0)) for t in dests])
-    row_end = J if row_end is None else row_end
-    with torch.cuda.device(dev):
-        native.call("sd_fisher_pairwise_scatter", J, S, native.ptr(inc), inc.stride(0), native.ptr(exc), exc.stride(0),
-                    P, native.ptr(pa), native.ptr(pb), n, ptrs, cols, lds, int(dest_row_offset), row_begin, row_end,
-                    int(max_cell_bound), _sp())
 
 
 def fisher_pairwise_host(inc, exc, pair_a, pair_b, out=None, device=0):

@@ -58,16 +58,9 @@ def sample_pairs(n_samples):
     return [(i, j) for i in range(n_samples - 1) for j in range(i + 1, n_samples)]
 
 
-def pairwise_pvalues(events, counts, clusters, device=0, correction="none", gpus=1):
-    """float64[len(events), n_pairs] two-sided Fisher p-values, pair order as ``sample_pairs``;
-    ``correction`` = 'none' | 'pairwise' | 'all' applies Benjamini-Hochberg on the device before
-    the matrix comes back (pairwise_fisher.py:182-191)."""
-    from . import ops
-    import torch
-    n_events, n_samples = counts.shape if counts.ndim == 2 else (0, 0)
-    pairs = sample_pairs(n_samples)
-    if n_events == 0 or not pairs:
-        return np.zeros((n_events, len(pairs)))
+def checked_counts(counts):
+    """int64 copy of a host inclusion-count matrix; ValueError on counts the device path cannot take."""
+    counts = np.asarray(counts)
     as_int = counts.astype(np.int64)
     if not np.array_equal(as_int, counts):
         # the reference sums the float rows first and lets scipy truncate the summed table
@@ -78,20 +71,37 @@ def pairwise_pvalues(events, counts, clusters, device=0, correction="none", gpus
         raise ValueError("All values in `table` must be nonnegative.")
     if (as_int >= 2 ** 31).any():
         raise ValueError("counts of 2^31 and above are not supported")
+    return as_int
+
+
+def fisher_inputs(counts_int, row_ptr, col_idx, device):
+    """Upload a checked count matrix (or row slab with its local CSR) and sum its exclusion counts on
+    ``device``: (inc, exc, pair_a, pair_b, bound) for ops.fisher_pairwise over every sample pair."""
+    from . import ops
+    inc = ops.upload_counts(counts_int, device)
+    exc = ops.quant_ps(inc, row_ptr, col_idx, want_f32=False, want_exc=True)["exc"]
+    pa, pb = ops.all_pairs(counts_int.shape[1])
+    # the host filled the matrix, so it can vouch for a bound on inc + exc: no reduction / sync on the device
+    bound = int(counts_int.max(initial=0)) * (1 + int(np.diff(row_ptr).max(initial=0)))
+    return inc, exc, pa, pb, bound
+
+
+def pairwise_pvalues(events, counts, clusters, device=0, correction="none", gpus=1):
+    """float64[len(events), n_pairs] two-sided Fisher p-values, pair order as ``sample_pairs``;
+    ``correction`` = 'none' | 'pairwise' | 'all' applies Benjamini-Hochberg on the device before
+    the matrix comes back (pairwise_fisher.py:182-191)."""
+    from . import ops
+    import torch
+    n_events, n_samples = counts.shape if counts.ndim == 2 else (0, 0)
+    n_pairs = n_samples * (n_samples - 1) // 2
+    if n_events == 0 or not n_pairs:
+        return np.zeros((n_events, n_pairs))
+    as_int = checked_counts(counts)
     row_ptr, col_idx = jn.csr_from_named_lists(events, clusters, "isin")
     if gpus > 1:                                    # one worker process per GPU (row slabs; NCCL for the correction)
         from . import multigpu
-        return multigpu.pairwise(as_int, row_ptr, col_idx, len(pairs), correction=correction, n_gpus=gpus)
-    dev = torch.device("cuda", device)
-    S = n_samples
-    buf = torch.zeros((n_events, (S + 3) // 4 * 4), dtype=torch.int32, device=dev)
-    buf[:, :S] = torch.from_numpy(as_int.astype(np.int32)).to(dev)
-    inc = buf[:, :S]
-    exc = ops.quant_ps(inc, row_ptr, col_idx, want_f32=False, want_exc=True)["exc"]
-    pa = np.array([a for a, _ in pairs], dtype=np.int32)
-    pb = np.array([b for _, b in pairs], dtype=np.int32)
-    # the host filled the matrix, so it can vouch for a bound on inc + exc: no reduction / sync on the device
-    bound = int(as_int.max(initial=0)) * (1 + int(np.diff(row_ptr).max(initial=0)))
+        return multigpu.pairwise(as_int, row_ptr, col_idx, n_pairs, correction=correction, n_gpus=gpus)
+    inc, exc, pa, pb, bound = fisher_inputs(as_int, row_ptr, col_idx, torch.device("cuda", device))
     p = ops.fisher_pairwise(inc, exc, pa, pb, max_cell_bound=bound)
     if correction != "none":
         ops.bh_adjust(p, correction, out=p)

@@ -141,8 +141,8 @@ def test_bounded_entry_point_matches_and_guards():
 def test_kernel_instantiations_agree():
     """Every instantiation of the pairwise kernel on the same tables: staged table (mode 0), table
     partly / wholly in global memory (modes 1, 2 with the Stirling fallback, chosen through the
-    promised bound), 64-bit totals (the pair-order kernel), the plain kernel by environment
-    switch -- and more than 512 samples, where the junction row is not staged in shared memory."""
+    promised bound), 64-bit totals (the pair-order kernel, bound 2^31) -- and more than 512
+    samples, where the junction row is not staged in shared memory."""
     import os
     _, ops = _ops()
     J, S = 700, 10
@@ -155,12 +155,6 @@ def test_kernel_instantiations_agree():
     for bound in (int((counts + exc).max()), 20_000, 3_000_000, 2 ** 31):
         got = ops.fisher_pairwise(inc_d, exc_d, pa, pb, max_cell_bound=bound).cpu().numpy()
         _check(got.ravel(), want.ravel(), rtol=1e-11)
-    os.environ["SD_FISHER_PLAIN"] = "1"
-    try:
-        got = ops.fisher_pairwise(inc_d, exc_d, pa, pb).cpu().numpy()
-    finally:
-        del os.environ["SD_FISHER_PLAIN"]
-    _check(got.ravel(), want.ravel(), rtol=1e-11)
     # per-sample log-factorial terms staged once per junction (the default whenever they fit next
     # to the table) against the same arithmetic evaluated per pair: identical bits; a table that
     # fills shared memory (bound 5,000 -> 10,001 entries) leaves no room for 400 samples' terms

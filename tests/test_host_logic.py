@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle_np
-from splicedice_b200 import counts_to_ps, ir_table, junctions as jn, pairwise_fisher
+from splicedice_b200 import counts_to_ps, ir_table, junctions as jn, ops, pairwise_fisher
 
 
 def test_names_round_trip():
@@ -54,6 +54,8 @@ def test_bh_oracle_known_values():
 
 def test_pair_order():
     assert pairwise_fisher.sample_pairs(4) == [(0, 1), (0, 2), (0, 3), (1, 2), (1, 3), (2, 3)]
+    for n in (0, 1, 2, 5, 13):              # the column header and the device pair arrays agree
+        assert pairwise_fisher.sample_pairs(n) == list(zip(*ops.all_pairs(n)))
 
 
 def test_parsers_on_reference_files(golden_dir):

@@ -226,6 +226,24 @@ int sd_peer_scatter_rows(const double *src, int64_t n_rows, int64_t width, int32
 int sd_fisher_tables(int64_t n_tables, const int64_t *a, const int64_t *b,
                      const int64_t *c, const int64_t *d, double *p_out, void *stream);
 
+/* ---- K3 chi-squared: pairwise Yates-corrected chi-squared test ------------------------------
+ * Replaces the `--chi2` branch of the same loop: scipy.stats.chi2_contingency(table)[1] with its
+ * default correction=True (scipy 1.18.1, stats/contingency.py; pairwise_fisher.py:133-134,179).
+ * For rows j in [row_begin, row_end) and pairs k < n_pairs, on the same tables as sd_fisher_pairwise:
+ *   p_out[j, k] = erfc(sqrt(stat / 2)),  stat = max(|ad - bc| - N/2, 0)^2 N / (r1 r2 c1 c2)
+ * (p = 1 exactly where |ad - bc| <= N/2), NaN for the all-zero table (as scipy).  Tables scipy refuses
+ * -- a zero margin with N > 0, or an entry outside inc in [0, 2^31), exc in [0, 2^61) -- give NaN, and
+ * if first_refused (a DEVICE pointer, may be NULL) is set, *first_refused is lowered to the smallest
+ * j * n_pairs + k among them (j the absolute row); the caller initialises it to UINT64_MAX.  Fully
+ * asynchronous on `stream`: no scan, no synchronisation. */
+int sd_chi2_pairwise(int64_t n_junctions, int32_t n_samples,
+                     const int32_t *inc, int64_t ld_inc,
+                     const int64_t *exc, int64_t ld_exc,
+                     int64_t n_pairs, const int32_t *pair_a, const int32_t *pair_b,
+                     double *p_out, int64_t ld_p,
+                     int64_t row_begin, int64_t row_end,
+                     uint64_t *first_refused, void *stream);
+
 /* ---- Benjamini-Hochberg adjustment of the p-value matrix (device) ---------------------------
  * Replaces the multiple-test correction of pairwise_fisher.run_with (pairwise_fisher.py:182-191):
  * statsmodels multipletests(method="fdr_bh")[1] applied to every column ("pairwise", the CLI

@@ -310,24 +310,30 @@ def pairwise_fused(inc, exc, pair_a, pair_b, parts, bound, adjust=True):
     return rows.own
 
 
-def pairwise_sharded(counts_host, row_ptr, col_idx, correction="pairwise", device=None):
-    """``splicedice pairwise`` arithmetic over the ranks' GPUs: exclusion sums + Fisher on this
-    rank's row slab, then the correction.  counts_host: integer [J, S] on every rank (each uploads
-    only its slab).  Returns (float64 CUDA tensor [rows_r, P], (r0, r1))."""
+def pairwise_sharded(counts_host, row_ptr, col_idx, correction="pairwise", device=None, test="fisher", refused=None):
+    """``splicedice pairwise`` arithmetic over the ranks' GPUs: exclusion sums + Fisher (or the
+    chi-squared test, ``test='chi2'``) on this rank's row slab, then the correction.  counts_host:
+    integer [J, S] on every rank (each uploads only its slab).  Returns (float64 CUDA tensor
+    [rows_r, P], (r0, r1)).  chi2: ``refused`` as in ops.chi2_pairwise, the index local to the slab."""
     from . import ops
     from .pairwise_fisher import checked_counts, fisher_inputs
     rank, world = _world()
     if correction not in ("none", "pairwise", "all"):
         raise ValueError("correction must be 'none', 'pairwise' or 'all'")
+    if test not in ("fisher", "chi2"):
+        raise ValueError("test must be 'fisher' or 'chi2'")
     dev = torch.device("cuda", torch.cuda.current_device() if device is None else device)
     parts = sharding.partition_rows(row_ptr, col_idx, world)
     r0, r1 = parts[rank]
     rp, ci = sharding.shard_csr(row_ptr, col_idx, r0, r1)
     inc, exc, pa, pb, bound = fisher_inputs(checked_counts(counts_host[r0:r1]), rp, ci, dev)
-    if correction == "pairwise" and 1 < world <= FUSED_MAX_WORLD and dist.get_backend() == "nccl" and len(pa) >= world:
+    if test == "chi2":                               # the NCCL exchange below: no fused scatter form
+        p = ops.chi2_pairwise(inc, exc, pa, pb, refused=refused)
+    elif correction == "pairwise" and 1 < world <= FUSED_MAX_WORLD and dist.get_backend() == "nccl" and len(pa) >= world:
         # the exchange rides on the kernels' own stores (peer memory); see pairwise_fused
         return pairwise_fused(inc, exc, pa, pb, parts, bound).clone(), (r0, r1)
-    p = ops.fisher_pairwise(inc, exc, pa, pb, max_cell_bound=bound)
+    else:
+        p = ops.fisher_pairwise(inc, exc, pa, pb, max_cell_bound=bound)
     if correction == "pairwise":
         p = bh_columns_sharded(p, parts, lambda cols: ops.bh_adjust(cols, "pairwise", out=cols))
     elif correction == "all":

@@ -86,7 +86,7 @@ def quant_ps(counts, row_ptr, col_idx, low_mask=None, n_gpus=2):
 
 
 # ---- pairwise -----------------------------------------------------------------------------------
-def _pairwise_worker(rank, world, port, counts, row_ptr, col_idx, correction, out):
+def _pairwise_worker(rank, world, port, counts, row_ptr, col_idx, correction, test, out, refused):
     import torch
     import torch.distributed as dist
     from . import distributed
@@ -94,18 +94,28 @@ def _pairwise_worker(rank, world, port, counts, row_ptr, col_idx, correction, ou
     dist.init_process_group("nccl", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=world,
                             device_id=torch.device("cuda", rank))
     try:
-        p, (r0, r1) = distributed.pairwise_sharded(counts.numpy(), row_ptr.numpy(), col_idx.numpy(), correction, device=rank)
+        # a rank that meets a refused chi-squared table still finishes every collective (the others would
+        # wait for it) and reports the table through shared memory
+        ref = torch.full((1,), -1, dtype=torch.int64, device=torch.device("cuda", rank)) if test == "chi2" else None
+        p, (r0, r1) = distributed.pairwise_sharded(counts.numpy(), row_ptr.numpy(), col_idx.numpy(), correction,
+                                                   device=rank, test=test, refused=ref)
         out[r0:r1] = p.cpu()
+        if ref is not None and int(ref.item()) != -1:
+            refused[rank] = int(ref.item()) + r0 * out.shape[1]
     finally:
         dist.destroy_process_group()
 
 
-def pairwise(counts_int, row_ptr, col_idx, n_pairs, correction="pairwise", n_gpus=2):
-    """float64[J, n_pairs] (corrected) p-values on ``n_gpus`` GPUs (distributed.pairwise_sharded)."""
+def pairwise(counts_int, row_ptr, col_idx, n_pairs, correction="pairwise", n_gpus=2, test="fisher"):
+    """(float64[J, n_pairs] (corrected) p-values, first refused index) on ``n_gpus`` GPUs
+    (distributed.pairwise_sharded).  The index is row * n_pairs + pair of the first table the
+    chi-squared test refuses (as sd_chi2_pairwise reports it on one GPU), None when there is none."""
     import torch
     n_gpus = check_gpus(n_gpus)
     J = counts_int.shape[0]
     out = torch.empty((J, n_pairs), dtype=torch.float64).share_memory_()
+    refused = torch.full((n_gpus,), -1, dtype=torch.int64).share_memory_()
     _spawn(_pairwise_worker, n_gpus, (_free_port(), _shared(counts_int, np.int64), _shared(row_ptr, np.int32),
-                                      _shared(col_idx, np.int32), correction, out))
-    return out.numpy()
+                                      _shared(col_idx, np.int32), correction, test, out, refused))
+    found = [int(v) for v in refused.tolist() if v != -1]
+    return out.numpy(), (min(found) if found else None)

@@ -67,6 +67,8 @@ _SIGNATURES = {
     "sd_fisher_pairwise_host": (c_int, [c_int, c_int64, c_int32, _P, c_int64, _P, c_int64,
                                         c_int64, _P, _P, _P, c_int64]),
     "sd_pairwise_host": (c_int, [c_int, c_int64, c_int32, _P, c_int64, _P, _P, c_int64, _P, _P, _P, c_int64]),
+    "sd_chi2_pairwise": (c_int, [c_int64, c_int32, _P, c_int64, _P, c_int64, c_int64, _P, _P,
+                                 _P, c_int64, c_int64, c_int64, _P, _P]),
     "sd_bh_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int]),
     "sd_bh_adjust": (c_int, [c_int64, c_int64, _P, c_int64, _P, c_int64, c_int, _P, c_size_t, _P]),
     "sd_ir_ratio": (c_int, [c_int64, c_int32, _P, c_int64, _P, c_int64, _P, _P, _P, c_int64,

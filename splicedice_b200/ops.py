@@ -190,6 +190,35 @@ def fisher_pairwise(inc, exc, pair_a, pair_b, row_begin=0, row_end=None, out=Non
     return out
 
 
+def chi2_pairwise(inc, exc, pair_a, pair_b, row_begin=0, row_end=None, out=None, refused=None):
+    """p[j, k] = Yates-corrected chi-squared p (scipy.stats.chi2_contingency(table)[1]) of the same
+    tables as fisher_pairwise (sd_chi2_pairwise; fully asynchronous).  Tables scipy refuses (a zero
+    margin with a non-zero total) give NaN; ``refused``, a one-element int64 CUDA tensor the caller sets
+    to -1, is lowered to the smallest j * n_pairs + k among them (read as uint64: -1 = none)."""
+    require_cuda()
+    if inc.dtype != torch.int32 or exc.dtype != torch.int64 or not inc.is_cuda or not exc.is_cuda:
+        raise TypeError("chi2_pairwise: inc int32 / exc int64 CUDA tensors expected")
+    if refused is not None and (refused.dtype != torch.int64 or refused.device != inc.device or refused.numel() != 1):
+        raise TypeError("chi2_pairwise: refused must be a one-element int64 tensor on the counts' device")
+    J, S = inc.shape
+    dev = inc.device
+    for arr in (pair_a, pair_b):
+        if not isinstance(arr, torch.Tensor):
+            h = np.asarray(arr)
+            if h.size and (h.min() < 0 or h.max() >= S):
+                raise ValueError("chi2_pairwise: pair index out of range")
+    pa, pb = _i32(pair_a, dev), _i32(pair_b, dev)
+    P = int(pa.numel())
+    row_end = J if row_end is None else row_end
+    if out is None:
+        out = torch.empty((J, P), dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        native.call("sd_chi2_pairwise", J, S, native.ptr(inc), inc.stride(0), native.ptr(exc), exc.stride(0), P,
+                    native.ptr(pa), native.ptr(pb), native.ptr(out), out.stride(0), row_begin, row_end,
+                    native.ptr(refused), _sp())
+    return out
+
+
 def fisher_pairwise_host(inc, exc, pair_a, pair_b, out=None, device=0):
     require_cuda()
     inc = np.ascontiguousarray(inc, dtype=np.int32) if not isinstance(inc, torch.Tensor) else inc

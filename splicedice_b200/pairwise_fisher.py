@@ -1,11 +1,11 @@
-"""``splicedice pairwise`` on a B200: per-event Fisher exact test for every sample pair.
+"""``splicedice pairwise`` on a B200: per-event Fisher exact (or ``--chi2``) test for every sample pair.
 
 Host mirror of /root/reference/splicedice/pairwise_fisher.py (same flags, inputs and output
 file).  The hot loop (pairwise_fisher.py:154-180) runs on the GPU: exclusion counts with
-sd_quant_ps over the cluster CSR, then sd_fisher_pairwise for the [events x pairs] p-values.
-Benjamini-Hochberg runs on the device too (sd_bh_adjust); the writer is the native host
-formatter.  ``--chi2`` is not implemented (out of scope: BASELINE.json names the Fisher path
-only) and is rejected loudly.
+sd_quant_ps over the cluster CSR, then sd_fisher_pairwise (or sd_chi2_pairwise) for the
+[events x pairs] p-values.  Benjamini-Hochberg runs on the device too (sd_bh_adjust); the writer
+is the native host formatter.  With ``--chi2`` a table scipy's chi2_contingency refuses (a zero
+margin) raises the same ValueError the reference's loop stops on, and no file is written.
 """
 from __future__ import annotations
 
@@ -86,12 +86,39 @@ def fisher_inputs(counts_int, row_ptr, col_idx, device):
     return inc, exc, pa, pb, bound
 
 
-def pairwise_pvalues(events, counts, clusters, device=0, correction="none", gpus=1):
-    """float64[len(events), n_pairs] two-sided Fisher p-values, pair order as ``sample_pairs``;
-    ``correction`` = 'none' | 'pairwise' | 'all' applies Benjamini-Hochberg on the device before
-    the matrix comes back (pairwise_fisher.py:182-191)."""
+def chi2_refusal(first, counts_int, row_ptr, col_idx, events, samples=None):
+    """ValueError for the first table scipy.stats.chi2_contingency refuses, ``first`` = row * n_pairs +
+    pair (sd_chi2_pairwise's index): scipy's message with the (i, j) of the first zero expected frequency,
+    then the event, the ``a_b`` column and the table.  The table is rebuilt on the host from the CSR."""
+    pa, pb = np.triu_indices(counts_int.shape[1], k=1)          # the pair order of ops.all_pairs
+    j, k = divmod(int(first), len(pa))
+    sa, sb = int(pa[k]), int(pb[k])
+    members = col_idx[row_ptr[j]:row_ptr[j + 1]]
+    a, b = int(counts_int[j, sa]), int(counts_int[j, sb])
+    c, d = int(counts_int[members, sa].sum()), int(counts_int[members, sb].sum())
+    column = f"{samples[sa]}_{samples[sb]}" if samples is not None else f"{sa}_{sb}"
+    where = f"event {events[j]}, column {column}, table [[{a}, {b}], [{c}, {d}]]"
+    if a + b == 0 or a + c == 0:
+        pos = "(0, 0)"
+    elif b + d == 0:
+        pos = "(0, 1)"
+    elif c + d == 0:
+        pos = "(1, 0)"
+    else:
+        return ValueError(f"chi-squared test: table outside the supported range ({where})")
+    return ValueError(f"The internally computed table of expected frequencies has a zero element at {pos}. ({where})")
+
+
+def pairwise_pvalues(events, counts, clusters, device=0, correction="none", gpus=1, test="fisher", samples=None):
+    """float64[len(events), n_pairs] p-values, pair order as ``sample_pairs``: two-sided Fisher
+    (``test='fisher'``) or Yates-corrected chi-squared (``test='chi2'``, scipy's chi2_contingency; a
+    refused table raises ValueError naming the event and the column, from ``samples`` when given);
+    ``correction`` = 'none' | 'pairwise' | 'all' applies Benjamini-Hochberg on the device before the
+    matrix comes back (pairwise_fisher.py:182-191)."""
     from . import ops
     import torch
+    if test not in ("fisher", "chi2"):
+        raise ValueError("test must be 'fisher' or 'chi2'")
     n_events, n_samples = counts.shape if counts.ndim == 2 else (0, 0)
     n_pairs = n_samples * (n_samples - 1) // 2
     if n_events == 0 or not n_pairs:
@@ -100,9 +127,19 @@ def pairwise_pvalues(events, counts, clusters, device=0, correction="none", gpus
     row_ptr, col_idx = jn.csr_from_named_lists(events, clusters, "isin")
     if gpus > 1:                                    # one worker process per GPU (row slabs; NCCL for the correction)
         from . import multigpu
-        return multigpu.pairwise(as_int, row_ptr, col_idx, n_pairs, correction=correction, n_gpus=gpus)
+        p, first = multigpu.pairwise(as_int, row_ptr, col_idx, n_pairs, correction=correction, n_gpus=gpus, test=test)
+        if first is not None:
+            raise chi2_refusal(first, as_int, row_ptr, col_idx, events, samples)
+        return p
     inc, exc, pa, pb, bound = fisher_inputs(as_int, row_ptr, col_idx, torch.device("cuda", device))
-    p = ops.fisher_pairwise(inc, exc, pa, pb, max_cell_bound=bound)
+    if test == "chi2":
+        refused = torch.full((1,), -1, dtype=torch.int64, device=inc.device)
+        p = ops.chi2_pairwise(inc, exc, pa, pb, refused=refused)
+        first = int(refused.item())
+        if first != -1:                             # the reference's loop stops at this table
+            raise chi2_refusal(first, as_int, row_ptr, col_idx, events, samples)
+    else:
+        p = ops.fisher_pairwise(inc, exc, pa, pb, max_cell_bound=bound)
     if correction != "none":
         ops.bh_adjust(p, correction, out=p)
     return p.cpu().numpy()
@@ -113,7 +150,7 @@ def add_parser(parser):
                         help="inclusionCounts.tsv written by quant")
     parser.add_argument("-c", "--clusters", type=str, required=True, help="allClusters.tsv written by quant")
     parser.add_argument("--chi2", action="store_true", default=False,
-                        help="(reference flag) chi-squared instead of Fisher -- not available on the GPU path")
+                        help="Yates-corrected chi-squared test (scipy's chi2_contingency) instead of Fisher")
     parser.add_argument("--multiple_test_correction", default="pairwise", choices=["pairwise", "all", "none"],
                         help="Benjamini-Hochberg per sample pair (default), over all p-values, or none")
     parser.add_argument("-f", "--filter_list", help="text file of events to analyse, one per line")
@@ -124,8 +161,6 @@ def add_parser(parser):
 
 
 def run_with(args):
-    if args.chi2:
-        raise NotImplementedError("--chi2 is outside the B200 hot path (Fisher only); use the reference for it")
     filter_list = None
     if args.filter_list is not None:
         with open(args.filter_list) as handle:
@@ -139,7 +174,8 @@ def run_with(args):
     print("Analyzing pairs:")
     print(",".join(columns))
     parray = pairwise_pvalues(events, counts, clusters, getattr(args, "device", 0),
-                              correction=args.multiple_test_correction, gpus=getattr(args, "gpus", 1))
+                              correction=args.multiple_test_correction, gpus=getattr(args, "gpus", 1),
+                              test="chi2" if args.chi2 else "fisher", samples=samples)
     print(f"[{len(events)} / {len(events)}] events analyzed...")
     from . import textio
     textio.write_matrix(args.output, "clusterID\t" + "\t".join(columns) + "\n", events,
@@ -148,6 +184,6 @@ def run_with(args):
 
 if __name__ == "__main__":
     import argparse
-    cli = argparse.ArgumentParser(description="pairwise Fisher exact tests (B200)")
+    cli = argparse.ArgumentParser(description="pairwise Fisher exact / chi-squared tests (B200)")
     add_parser(cli)
     run_with(cli.parse_args())

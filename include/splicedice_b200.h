@@ -266,6 +266,28 @@ int sd_bh_adjust(int64_t n_rows, int64_t n_cols, const double *p, int64_t ld_p,
                  double *out, int64_t ld_out, int mode,
                  void *workspace, size_t workspace_bytes, void *stream);
 
+/* ---- K6: Wilcoxon rank-sum test per event between two sample groups (compare_groups) ------------
+ * For rows j in [row_begin, row_end) of the PS matrix ps[n_events, n_samples] (float32 or float64 by
+ * `dtype`; NaN = undefined cell): x = the non-NaN cells of columns cols1[0, n1), y = those of
+ * cols2[0, n2) (DEVICE int32 lists; the caller keeps the groups disjoint), and
+ *   n_out[j * ld_n + 0, 1]            = |x|, |y|
+ *   stats_out[j * ld_stats + 0 .. 3]  = mean(x), mean(y), z, p
+ * with z, p = scipy.stats.ranksums(x, y, nan_policy='omit') (scipy 1.18.1): average ranks for ties, no
+ * tie or continuity correction, p = erfc(|z| / sqrt 2).  2 R1 - n1 (n + 1) is exact in 64-bit
+ * integers, so balanced rank sums give z == 0 and p == 1 exactly.  -0.0 ties +0.0; +-inf are ordinary
+ * values; means are float64 sums.  An empty x or y gives NaN z, p and NaN for that group's mean.
+ * n1, n2 >= 1 and n1 + n2 <= SD_RANKSUM_MAX_SAMPLES (the sort runs in shared memory).  A column index
+ * outside [0, n_samples) is never read: the rows get n = -1 and NaN statistics.  One asynchronous
+ * launch on `stream`, no synchronisation.
+ */
+#define SD_RANKSUM_F32 0
+#define SD_RANKSUM_F64 1
+#define SD_RANKSUM_MAX_SAMPLES 16384
+int sd_ranksum_rows(int64_t n_events, int32_t n_samples, const void *ps, int64_t ld_ps, int dtype,
+                    int32_t n1, const int32_t *cols1, int32_t n2, const int32_t *cols2,
+                    int64_t row_begin, int64_t row_end,
+                    int32_t *n_out, int64_t ld_n, double *stats_out, int64_t ld_stats, void *stream);
+
 /* ---- K4: intron-retention ratio ----------------------------------------------------
  * Replaces the arithmetic of ir_table.calculateIR (ir_table.py:118-132):
  *   ir[r,s] = median[r,s] / (median[r,s] + inc[r,s] + sum_{c in adj(r)} inc[c,s]),  x/0 -> NaN

@@ -1,15 +1,17 @@
 """``python -m splicedice_b200 <command>``: the hot-path commands of the splicedice CLI
-(quant, counts_to_ps, pairwise, ir_table) with the reference's flags, running on a B200.
-The remaining reference commands (BAM readers, downstream statistics) are out of scope."""
+(quant, counts_to_ps, pairwise, ir_table) with the reference's flags, and compare_groups (a
+rank-sum test per event between two sample groups), running on a B200.
+The remaining reference commands (BAM readers, the other downstream statistics) are out of scope."""
 import argparse
 
-from . import counts_to_ps, ir_table, pairwise_fisher, quant
+from . import compare_groups, counts_to_ps, ir_table, pairwise_fisher, quant
 
 COMMANDS = {
     "quant": quant,
     "counts_to_ps": counts_to_ps,
     "pairwise": pairwise_fisher,
     "ir_table": ir_table,
+    "compare_groups": compare_groups,
 }
 
 

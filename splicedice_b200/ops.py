@@ -306,6 +306,54 @@ def fisher_tables(a, b, c, d, device=None):
 
 
 # ---------------------------------------------------------------------------------------
+# K6
+# ---------------------------------------------------------------------------------------
+def ranksum_rows(ps, cols1, cols2, row_begin=0, row_end=None, out=None):
+    """Wilcoxon rank-sum test per row between two column groups of a float32 / float64 CUDA PS matrix
+    (sd_ranksum_rows; fully asynchronous): scipy.stats.ranksums(x, y, nan_policy='omit') on the non-NaN
+    cells x of ``cols1`` and y of ``cols2``.  Returns a dict of [J] CUDA views n1, n2 (int32) and mean1,
+    mean2, z, p (float64); only rows [row_begin, row_end) are written.  ``out`` = (int32 [J, >= 2],
+    float64 [J, >= 4]) gives the buffers behind those views.  Host column lists are checked here
+    (integers in [0, S), each group non-empty and without repeats, the groups disjoint); CUDA int32
+    tensors are taken as they are (the kernel never reads a column outside [0, S))."""
+    require_cuda()
+    if ps.dtype not in (torch.float32, torch.float64) or not ps.is_cuda or ps.dim() != 2:
+        raise TypeError("ranksum_rows: ps must be a 2-D float32 / float64 CUDA tensor")
+    J, S = ps.shape
+    if J and S and ps.stride(1) != 1:
+        raise ValueError("ranksum_rows: ps must be row-major")
+    dev = ps.device
+    host = {}
+    for name, cols in (("cols1", cols1), ("cols2", cols2)):
+        if isinstance(cols, torch.Tensor) and cols.is_cuda:
+            continue
+        h = np.asarray(cols.cpu() if isinstance(cols, torch.Tensor) else cols)
+        if h.ndim != 1 or h.size == 0 or not np.issubdtype(h.dtype, np.integer):
+            raise ValueError(f"ranksum_rows: {name} must be a non-empty list of column indices")
+        if h.min() < 0 or h.max() >= S:
+            raise ValueError(f"ranksum_rows: {name} has a column outside [0, {S})")
+        if np.unique(h).size != h.size:
+            raise ValueError(f"ranksum_rows: {name} lists a column twice")
+        host[name] = h
+    if len(host) == 2 and np.intersect1d(host["cols1"], host["cols2"]).size:
+        raise ValueError("ranksum_rows: cols1 and cols2 share a column")
+    c1, c2 = _i32(cols1, dev), _i32(cols2, dev)
+    row_end = J if row_end is None else row_end
+    if out is None:
+        out = (torch.empty((J, 2), dtype=torch.int32, device=dev), torch.empty((J, 4), dtype=torch.float64, device=dev))
+    n_out, st = out
+    if (n_out.dtype != torch.int32 or st.dtype != torch.float64 or n_out.device != dev or st.device != dev
+            or n_out.shape[0] != J or st.shape[0] != J or n_out.stride(1) != 1 or st.stride(1) != 1):
+        raise TypeError("ranksum_rows: out must be (int32 [J, >= 2], float64 [J, >= 4]) on the PS device")
+    kind = native.SD_RANKSUM_F32 if ps.dtype == torch.float32 else native.SD_RANKSUM_F64
+    with torch.cuda.device(dev):
+        native.call("sd_ranksum_rows", J, S, native.ptr(ps), ps.stride(0), kind, c1.numel(), native.ptr(c1),
+                    c2.numel(), native.ptr(c2), row_begin, row_end, native.ptr(n_out), n_out.stride(0),
+                    native.ptr(st), st.stride(0), _sp())
+    return dict(n1=n_out[:, 0], n2=n_out[:, 1], mean1=st[:, 0], mean2=st[:, 1], z=st[:, 2], p=st[:, 3])
+
+
+# ---------------------------------------------------------------------------------------
 # K4
 # ---------------------------------------------------------------------------------------
 def ir_ratio(median, counts, row_ptr=None, col_idx=None, row_begin=0, row_end=None):

@@ -288,6 +288,29 @@ int sd_ranksum_rows(int64_t n_events, int32_t n_samples, const void *ps, int64_t
                     int64_t row_begin, int64_t row_end,
                     int32_t *n_out, int64_t ld_n, double *stats_out, int64_t ld_stats, void *stream);
 
+/* ---- K7: Kruskal-Wallis H test per event across sample groups (compare_conditions) ---------------
+ * For rows j in [row_begin, row_end) of ps (as K6): the non-NaN cells of columns cols[0, n_cols), the
+ * cell of cols[i] in group group_of[i] (DEVICE int32 lists; columns listed once), ranked together with
+ * average ranks, and
+ *   n_out[j * ld_n + g]              = defined cells of group g, g < n_groups
+ *   mean_out[j * ld_mean + g]        = their mean (float64 sum; NaN for an empty group)
+ *   stats_out[j * ld_stats + 0, 1]   = H, p
+ * with H, p = scipy.stats.kruskal(*groups, nan_policy='omit') (scipy 1.18.1) computed without its
+ * cancellation: H = 3 (n - 1) sum_g (D_g^2 / n_g) / (n^3 - n - T), D_g = 2 R_g - n_g (n + 1) and the tie
+ * term T exact in 64-bit integers, p = chi2.sf(H, n_groups - 1).  H >= 0, and balanced rank sums give
+ * H == 0 and p == 1 exactly.  An empty group, or every defined cell tied, gives H = p = NaN (scipy gives
+ * NaN for the first, NaN or +-inf for the second).  -0.0 ties +0.0; +-inf are ordinary values.
+ * 2 <= n_groups <= SD_KRUSKAL_MAX_GROUPS, 1 <= n_cols <= SD_RANKSUM_MAX_SAMPLES.  A column outside
+ * [0, n_samples) or a label outside [0, n_groups) is never dereferenced: the rows get n = -1 in every
+ * group and NaN means and statistics.  One asynchronous launch on `stream`, no synchronisation.
+ */
+#define SD_KRUSKAL_MAX_GROUPS 256
+int sd_kruskal_rows(int64_t n_events, int32_t n_samples, const void *ps, int64_t ld_ps, int dtype,
+                    int32_t n_groups, int32_t n_cols, const int32_t *cols, const int32_t *group_of,
+                    int64_t row_begin, int64_t row_end,
+                    int32_t *n_out, int64_t ld_n, double *mean_out, int64_t ld_mean,
+                    double *stats_out, int64_t ld_stats, void *stream);
+
 /* ---- K4: intron-retention ratio ----------------------------------------------------
  * Replaces the arithmetic of ir_table.calculateIR (ir_table.py:118-132):
  *   ir[r,s] = median[r,s] / (median[r,s] + inc[r,s] + sum_{c in adj(r)} inc[c,s]),  x/0 -> NaN

@@ -1,10 +1,11 @@
 """``python -m splicedice_b200 <command>``: the hot-path commands of the splicedice CLI
-(quant, counts_to_ps, pairwise, ir_table) with the reference's flags, and compare_groups (a
-rank-sum test per event between two sample groups), running on a B200.
+(quant, counts_to_ps, pairwise, ir_table) with the reference's flags, compare_groups (a rank-sum
+test per event between two sample groups) and compare_conditions (a Kruskal-Wallis test per event
+across any number of sample groups), running on a B200.
 The remaining reference commands (BAM readers, the other downstream statistics) are out of scope."""
 import argparse
 
-from . import compare_groups, counts_to_ps, ir_table, pairwise_fisher, quant
+from . import compare_conditions, compare_groups, counts_to_ps, ir_table, pairwise_fisher, quant
 
 COMMANDS = {
     "quant": quant,
@@ -12,6 +13,7 @@ COMMANDS = {
     "pairwise": pairwise_fisher,
     "ir_table": ir_table,
     "compare_groups": compare_groups,
+    "compare_conditions": compare_conditions,
 }
 
 

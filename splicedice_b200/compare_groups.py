@@ -67,6 +67,19 @@ def group_columns(samples, group1, group2):
     return cols[0], cols[1]
 
 
+def bh_over_tested(p):
+    """Benjamini-Hochberg ("all" mode, sd_bh_adjust) over the tested events of a CUDA p-value vector:
+    the events with a p-value; NaN where p is NaN."""
+    import torch
+
+    from . import ops
+    tested = torch.nonzero(~torch.isnan(p)).reshape(-1)
+    corrected = torch.full_like(p, float("nan"))
+    if tested.numel():
+        corrected[tested] = ops.bh_adjust(p[tested].reshape(-1, 1).contiguous(), "all").reshape(-1)
+    return corrected
+
+
 def compare(ps, cols1, cols2, device=0):
     """float64 [J, 6] = mean1, mean2, delta, z, pvalue, corrected for a host PS matrix (float32 or
     float64), BH over the events with a finite p only."""
@@ -80,10 +93,7 @@ def compare(ps, cols1, cols2, device=0):
     dev = torch.device("cuda", device)
     r = ops.ranksum_rows(torch.from_numpy(ps).to(dev), cols1, cols2)
     p = r["p"]
-    tested = torch.nonzero(~torch.isnan(p)).reshape(-1)
-    corrected = torch.full_like(p, float("nan"))
-    if tested.numel():
-        corrected[tested] = ops.bh_adjust(p[tested].reshape(-1, 1).contiguous(), "all").reshape(-1)
+    corrected = bh_over_tested(p)
     out[:, 0] = r["mean1"].cpu().numpy()
     out[:, 1] = r["mean2"].cpu().numpy()
     out[:, 2] = out[:, 0] - out[:, 1]

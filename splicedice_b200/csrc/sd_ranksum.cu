@@ -13,10 +13,8 @@
 // rounds exactly where scipy's float expression does (its rank sum of half-integers below 2^53 is
 // exact too), and D == 0 gives z == 0 and p == 1 exactly.
 //
-// Keys: the IEEE bit pattern made order-preserving (sign set: all bits flipped; clear: sign bit set),
-// after -0.0 is canonicalised to +0.0 (rankdata ties them).  float32 cells are widened to double first
-// (exact and order-preserving), so both input types share one key and one kernel body.  +-inf are
-// ordinary keys; ~0 pads the sort above every key a non-NaN value can have.
+// Keys, gather, sort and searches are the shared ones of sd_ranksort.cuh: -0.0 ties +0.0, float32 cells
+// are widened to double first, so both input types share one kernel body, and +-inf are ordinary keys.
 //
 // Mapping: one CTA per row (rows blockIdx.x, + gridDim.x, ...; one resident wave).  Gather the group
 // columns into shared memory with warp-aggregated slots, bitonic sort of the next power of two above
@@ -27,6 +25,7 @@
 #include <algorithm>
 
 #include "sd_common.cuh"
+#include "sd_ranksort.cuh"
 
 namespace sd {
 namespace ranksum {
@@ -34,7 +33,6 @@ namespace ranksum {
 constexpr int kMaxN = SD_RANKSUM_MAX_SAMPLES;
 constexpr int kMaxThreads = 256;
 constexpr int kMaxWarps = kMaxThreads / 32;
-constexpr uint64_t kPad = ~0ull;
 
 struct Params {
     int32_t n_samples;
@@ -49,29 +47,8 @@ struct Params {
     int64_t row_begin, row_end;
 };
 
-__device__ __forceinline__ uint64_t order_key(double v)
-{
-    uint64_t u = (uint64_t)__double_as_longlong(v);
-    if ((u << 1) == 0) u = 0;                                   // -0.0 -> +0.0
-    return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
-}
-
-// first position in keys[0, m) whose key is >= key (strict = false) or > key (strict = true)
-__device__ __forceinline__ int search(const uint64_t *keys, int lo, int m, uint64_t key, bool strict)
-{
-    int len = m - lo;
-    while (len > 0) {
-        const int half = len >> 1;
-        const uint64_t k = keys[lo + half];
-        if (k < key || (strict && k == key)) {
-            lo += half + 1;
-            len -= half + 1;
-        } else {
-            len = half;
-        }
-    }
-    return lo;
-}
+using ranksort::order_key;
+using ranksort::search;
 
 template <typename T>
 __global__ void __launch_bounds__(kMaxThreads) ranksum_rows_kernel(const Params p)
@@ -83,7 +60,6 @@ __global__ void __launch_bounds__(kMaxThreads) ranksum_rows_kernel(const Params 
     __shared__ int s_c1[kMaxWarps];
     const int n = p.n1 + p.n2;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const unsigned below = (1u << lane) - 1u;
     for (int64_t j = p.row_begin + blockIdx.x; j < p.row_end; j += gridDim.x) {
         const T *row = static_cast<const T *>(p.ps) + j * p.ld_ps;
         if (threadIdx.x == 0) {
@@ -116,11 +92,7 @@ __global__ void __launch_bounds__(kMaxThreads) ranksum_rows_kernel(const Params 
                     }
                 }
             }
-            const unsigned mask = __ballot_sync(0xffffffffu, valid);
-            int slot = 0;
-            if (lane == 0 && mask) slot = atomicAdd(&s_m, __popc(mask));
-            slot = __shfl_sync(0xffffffffu, slot, 0);
-            if (valid) keys[slot + __popc(mask & below)] = key;
+            SD_RANKSORT_APPEND(keys, &s_m, lane, valid, key);
         }
         __syncthreads();
         const int m = s_m;
@@ -134,24 +106,7 @@ __global__ void __launch_bounds__(kMaxThreads) ranksum_rows_kernel(const Params 
             __syncthreads();
             continue;
         }
-        int npad = 1;
-        while (npad < m) npad <<= 1;
-        for (int i = m + threadIdx.x; i < npad; i += blockDim.x) keys[i] = kPad;
-        __syncthreads();
-        // bitonic sort of keys[0, npad), ascending
-        for (int k = 2; k <= npad; k <<= 1) {
-            for (int h = k >> 1; h > 0; h >>= 1) {
-                for (int t = threadIdx.x; t < (npad >> 1); t += blockDim.x) {
-                    const int lo = 2 * t - (t & (h - 1)), hi = lo + h;
-                    const uint64_t a = keys[lo], b = keys[hi];
-                    if ((a > b) == ((lo & k) == 0)) {
-                        keys[lo] = b;
-                        keys[hi] = a;
-                    }
-                }
-                __syncthreads();
-            }
-        }
+        ranksort::sort(keys, m);
         // 2 R1 = sum over the group-1 cells of (lo + hi + 1), lo / hi the bounds of the cell's tie run
         long long r1 = 0;
         for (int i = threadIdx.x; i < p.n1; i += blockDim.x) {

@@ -354,6 +354,62 @@ def ranksum_rows(ps, cols1, cols2, row_begin=0, row_end=None, out=None):
 
 
 # ---------------------------------------------------------------------------------------
+# K7
+# ---------------------------------------------------------------------------------------
+def kruskal_rows(ps, groups, row_begin=0, row_end=None, out=None):
+    """Kruskal-Wallis H test per row across the column groups ``groups`` (a list of k host column-index
+    lists) of a float32 / float64 CUDA PS matrix (sd_kruskal_rows; fully asynchronous):
+    scipy.stats.kruskal(*groups, nan_policy='omit') on the non-NaN cells, with NaN H and p where a group
+    has no defined cell or every defined cell is tied.  Returns a dict of CUDA views n (int32 [J, k]),
+    mean (float64 [J, k]), H and p (float64 [J]); only rows [row_begin, row_end) are written.
+    ``out`` = (int32 [J, >= k], float64 [J, >= k], float64 [J, >= 2]) gives the buffers behind those
+    views.  The lists are checked here: 2 <= k <= 256, each non-empty, integers in [0, S) without
+    repeats, the lists disjoint, at most 16,384 columns in all."""
+    require_cuda()
+    if ps.dtype not in (torch.float32, torch.float64) or not ps.is_cuda or ps.dim() != 2:
+        raise TypeError("kruskal_rows: ps must be a 2-D float32 / float64 CUDA tensor")
+    J, S = ps.shape
+    if J and S and ps.stride(1) != 1:
+        raise ValueError("kruskal_rows: ps must be row-major")
+    k = len(groups)
+    if not 2 <= k <= native.SD_KRUSKAL_MAX_GROUPS:
+        raise ValueError(f"kruskal_rows: {k} groups; 2 to {native.SD_KRUSKAL_MAX_GROUPS} are supported")
+    host = []
+    for g, cols in enumerate(groups):
+        h = np.asarray(cols.cpu() if isinstance(cols, torch.Tensor) else cols)
+        if h.ndim != 1 or h.size == 0 or not np.issubdtype(h.dtype, np.integer):
+            raise ValueError(f"kruskal_rows: group {g} must be a non-empty list of column indices")
+        if h.min() < 0 or h.max() >= S:
+            raise ValueError(f"kruskal_rows: group {g} has a column outside [0, {S})")
+        host.append(h.astype(np.int64))
+    cols = np.concatenate(host)
+    if cols.size > native.SD_RANKSUM_MAX_SAMPLES:
+        raise ValueError(f"kruskal_rows: {cols.size} columns in all; at most {native.SD_RANKSUM_MAX_SAMPLES}")
+    if np.unique(cols).size != cols.size:
+        raise ValueError("kruskal_rows: a column is listed twice")
+    dev = ps.device
+    # group by group, so that the lanes of a warp mostly share a label
+    group_of = np.repeat(np.arange(k, dtype=np.int32), [len(h) for h in host])
+    d_cols, d_group = _i32(cols, dev), _i32(group_of, dev)
+    row_end = J if row_end is None else row_end
+    if out is None:
+        out = (torch.empty((J, k), dtype=torch.int32, device=dev), torch.empty((J, k), dtype=torch.float64, device=dev),
+               torch.empty((J, 2), dtype=torch.float64, device=dev))
+    n_out, mean, st = out
+    if (n_out.dtype != torch.int32 or mean.dtype != torch.float64 or st.dtype != torch.float64
+            or any(t.dim() != 2 or t.device != dev or t.shape[0] != J or t.stride(1) != 1 for t in out)
+            or n_out.shape[1] < k or mean.shape[1] < k or st.shape[1] < 2):
+        raise TypeError("kruskal_rows: out must be (int32 [J, >= k], float64 [J, >= k], float64 [J, >= 2]) "
+                        "on the PS device")
+    kind = native.SD_RANKSUM_F32 if ps.dtype == torch.float32 else native.SD_RANKSUM_F64
+    with torch.cuda.device(dev):
+        native.call("sd_kruskal_rows", J, S, native.ptr(ps), ps.stride(0), kind, k, cols.size, native.ptr(d_cols),
+                    native.ptr(d_group), row_begin, row_end, native.ptr(n_out), n_out.stride(0), native.ptr(mean),
+                    mean.stride(0), native.ptr(st), st.stride(0), _sp())
+    return dict(n=n_out[:, :k], mean=mean[:, :k], H=st[:, 0], p=st[:, 1])
+
+
+# ---------------------------------------------------------------------------------------
 # K4
 # ---------------------------------------------------------------------------------------
 def ir_ratio(median, counts, row_ptr=None, col_idx=None, row_begin=0, row_end=None):

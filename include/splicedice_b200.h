@@ -311,6 +311,31 @@ int sd_kruskal_rows(int64_t n_events, int32_t n_samples, const void *ps, int64_t
                     int32_t *n_out, int64_t ld_n, double *mean_out, int64_t ld_mean,
                     double *stats_out, int64_t ld_stats, void *stream);
 
+/* ---- K8: Wilcoxon signed-rank test per event between matched sample pairs (compare_paired) -------
+ * For rows j in [row_begin, row_end) of ps (as K6): pair i has cells x_i = ps[j, cols1[i]] and
+ * y_i = ps[j, cols2[i]] (DEVICE int32 lists of n_pairs columns each; no column listed twice), and
+ *   n_out[j * ld_n + 0 .. 2]          = n, c, method
+ *   stats_out[j * ld_stats + 0 .. 3]  = mean1, mean2, W, p
+ * with W, p = scipy.stats.wilcoxon(x, y, nan_policy='omit') (scipy 1.18.1 defaults: zero_method
+ * 'wilcox', no continuity correction, two-sided, method 'auto').  n = pairs with both cells non-NaN
+ * (a pair with a NaN cell is dropped); d_i = x_i - y_i is subtracted in the input's precision and then
+ * widened; inf - inf counts in n but carries no rank; zeros (-0.0 included) are dropped; c = the
+ * remaining differences, ranked by |d| with average ranks.  2 R+ and the tie term are exact in 64-bit
+ * integers and W = min(R+, R-).  method 1 (n <= 50 without ties or zeros, or n <= 13): p is the exact
+ * sign-flip distribution of the c doubled ranks counted in 64-bit integers, bit-identical to scipy;
+ * method 2 (otherwise): the normal approximation with tie correction, z bit-identical to scipy and
+ * p = erfc(|z| / sqrt 2).  method 0 (untested: n = 0, n = 1 with a zero difference, or method 2 with
+ * c = 0): W = p = NaN.  mean1 / mean2 are float64 means of x and y over the n pairs (NaN for n = 0).
+ * 1 <= n_pairs <= SD_SIGNEDRANK_MAX_PAIRS (the sort runs in shared memory).  A column outside
+ * [0, n_samples) is never read: the rows get n = c = -1, method 0 and NaN statistics.  One asynchronous
+ * launch on `stream`, no synchronisation.
+ */
+#define SD_SIGNEDRANK_MAX_PAIRS 8192
+int sd_signedrank_rows(int64_t n_events, int32_t n_samples, const void *ps, int64_t ld_ps, int dtype,
+                       int32_t n_pairs, const int32_t *cols1, const int32_t *cols2,
+                       int64_t row_begin, int64_t row_end,
+                       int32_t *n_out, int64_t ld_n, double *stats_out, int64_t ld_stats, void *stream);
+
 /* ---- K4: intron-retention ratio ----------------------------------------------------
  * Replaces the arithmetic of ir_table.calculateIR (ir_table.py:118-132):
  *   ir[r,s] = median[r,s] / (median[r,s] + inc[r,s] + sum_{c in adj(r)} inc[c,s]),  x/0 -> NaN

@@ -410,6 +410,57 @@ def kruskal_rows(ps, groups, row_begin=0, row_end=None, out=None):
 
 
 # ---------------------------------------------------------------------------------------
+# K8
+# ---------------------------------------------------------------------------------------
+def signedrank_rows(ps, cols1, cols2, row_begin=0, row_end=None, out=None):
+    """Wilcoxon signed-rank test per row between matched column pairs (cols1[i], cols2[i]) of a float32 /
+    float64 CUDA PS matrix (sd_signedrank_rows; fully asynchronous): scipy.stats.wilcoxon(x, y,
+    nan_policy='omit') with the differences taken in the matrix's precision.  Returns a dict of [J] CUDA
+    views n, c, method (int32: complete pairs, ranked differences, 0 untested / 1 exact / 2 normal
+    approximation) and mean1, mean2, W, p (float64); only rows [row_begin, row_end) are written.
+    ``out`` = (int32 [J, >= 3], float64 [J, >= 4]) gives the buffers behind those views.  The lists are
+    checked here: the same non-zero length up to 8,192, integers in [0, S), no column listed twice in
+    either list or across both."""
+    require_cuda()
+    if ps.dtype not in (torch.float32, torch.float64) or not ps.is_cuda or ps.dim() != 2:
+        raise TypeError("signedrank_rows: ps must be a 2-D float32 / float64 CUDA tensor")
+    J, S = ps.shape
+    if J and S and ps.stride(1) != 1:
+        raise ValueError("signedrank_rows: ps must be row-major")
+    host = []
+    for name, cols in (("cols1", cols1), ("cols2", cols2)):
+        h = np.asarray(cols.cpu() if isinstance(cols, torch.Tensor) else cols)
+        if h.ndim != 1 or h.size == 0 or not np.issubdtype(h.dtype, np.integer):
+            raise ValueError(f"signedrank_rows: {name} must be a non-empty list of column indices")
+        if h.min() < 0 or h.max() >= S:
+            raise ValueError(f"signedrank_rows: {name} has a column outside [0, {S})")
+        host.append(h)
+    if host[0].size != host[1].size:
+        raise ValueError(f"signedrank_rows: cols1 has {host[0].size} columns, cols2 {host[1].size}; pairs need both")
+    if host[0].size > native.SD_SIGNEDRANK_MAX_PAIRS:
+        raise ValueError(f"signedrank_rows: {host[0].size} pairs; at most {native.SD_SIGNEDRANK_MAX_PAIRS}")
+    if np.unique(np.concatenate(host)).size != 2 * host[0].size:
+        raise ValueError("signedrank_rows: a column is listed twice")
+    dev = ps.device
+    c1, c2 = _i32(host[0], dev), _i32(host[1], dev)
+    row_end = J if row_end is None else row_end
+    if out is None:
+        out = (torch.empty((J, 3), dtype=torch.int32, device=dev), torch.empty((J, 4), dtype=torch.float64, device=dev))
+    n_out, st = out
+    if (n_out.dtype != torch.int32 or st.dtype != torch.float64
+            or any(t.dim() != 2 or t.device != dev or t.shape[0] != J or t.stride(1) != 1 for t in out)
+            or n_out.shape[1] < 3 or st.shape[1] < 4):
+        raise TypeError("signedrank_rows: out must be (int32 [J, >= 3], float64 [J, >= 4]) on the PS device")
+    kind = native.SD_RANKSUM_F32 if ps.dtype == torch.float32 else native.SD_RANKSUM_F64
+    with torch.cuda.device(dev):
+        native.call("sd_signedrank_rows", J, S, native.ptr(ps), ps.stride(0), kind, c1.numel(), native.ptr(c1),
+                    native.ptr(c2), row_begin, row_end, native.ptr(n_out), n_out.stride(0), native.ptr(st),
+                    st.stride(0), _sp())
+    return dict(n=n_out[:, 0], c=n_out[:, 1], method=n_out[:, 2], mean1=st[:, 0], mean2=st[:, 1], W=st[:, 2],
+                p=st[:, 3])
+
+
+# ---------------------------------------------------------------------------------------
 # K4
 # ---------------------------------------------------------------------------------------
 def ir_ratio(median, counts, row_ptr=None, col_idx=None, row_begin=0, row_end=None):

@@ -66,7 +66,10 @@ int sd_device_info(int device, int *sm_count, int *cc_major, int *cc_minor, size
  * as the reference's: priors most-recent-first, then laters ascending, :247-254).  The
  * build workspace must be passed, untouched, to sd_cluster_fill together with a second
  * workspace sized by sd_cluster_fill_workspace_bytes(n_junctions, nnz).
- * Preconditions: 0 <= start, end < 2^31; chrom_rank < 2^25; strand_rank < 2^8.
+ * Input domain: 0 <= start, end; 0 <= chrom_rank < 2^25; 0 <= strand_rank < 2^8.
+ * sd_cluster_build checks it on the device and refuses a junction outside it with
+ * SD_ERR_INVALID (reported at the call's read-back; the output arrays then hold
+ * unspecified values and nothing outside them and the workspace is written).
  *
  *   cluster_order[pos] = input index of the junction at position pos of cluster order
  *   out_row[i]         = output row of input junction i

@@ -41,15 +41,29 @@ __device__ __forceinline__ uint64_t seg_key(int32_t chrom, int32_t strand, int32
     return ((uint64_t)(uint32_t)chrom << 39) | ((uint64_t)(uint32_t)(strand & 0xFF) << 31) | (uint64_t)(uint32_t)coord;
 }
 
+// bits of the build's flag word (workspace `misc`, read back once per attempt)
+constexpr int32_t kFlagLongRun = 1;        // a run of equal keys is longer than kMaxRun: repeat with the two-pass sort
+constexpr int32_t kFlagBadInput = 2;       // a field lies outside what seg_key can pack: the call is refused
+
 __global__ void k_iota_end(int64_t n, const int32_t *end, uint32_t *key, int32_t *val)
 {
     SD_GRID_STRIDE(i, n) { key[i] = (uint32_t)end[i]; val[i] = (int32_t)i; }
 }
-// (chrom, strand, start) key of every junction in input order
-__global__ void k_key_direct(int64_t n, const int32_t *chrom, const int32_t *strand, const int32_t *start, uint64_t *key,
-                             int32_t *val)
+// (chrom, strand, start) key of every junction in input order.  Also the input check of the build:
+// a junction that seg_key would alias onto another key (chrom >= 2^25 or negative, strand outside
+// [0, 256), a negative start or end, whose bit 31 would land in the strand field) raises
+// kFlagBadInput.  The build only runs a second attempt after this one was read back clean, so the
+// second attempt's key kernel needs no check of its own.
+__global__ void k_key_direct(int64_t n, const int32_t *chrom, const int32_t *strand, const int32_t *start,
+                             const int32_t *end, uint64_t *key, int32_t *val, int32_t *flag)
 {
-    SD_GRID_STRIDE(i, n) { key[i] = seg_key(chrom[i], strand[i], start[i]); val[i] = (int32_t)i; }
+    SD_GRID_STRIDE(i, n)
+    {
+        const int32_t c = chrom[i], s = strand[i], st = start[i];
+        if ((uint32_t)c >= (1u << 25) || (uint32_t)s >= 256u || (st | end[i]) < 0) atomicOr(flag, kFlagBadInput);
+        key[i] = seg_key(c, s, st);
+        val[i] = (int32_t)i;
+    }
 }
 // After ONE sort by (chrom, strand, start): junctions that share all three (a common donor site)
 // form short runs that still have to be ordered by `end`.  The thread at the head of a run sorts
@@ -65,7 +79,7 @@ __global__ void k_fix_ties(int64_t n, const uint64_t *key_sorted, int32_t *order
         int64_t j = i + 2;
         while (j < n && j - i <= kMaxRun && key_sorted[j] == key) ++j;
         const int len = (int)(j - i);
-        if (len > kMaxRun) { atomicExch(flag, 1); continue; }
+        if (len > kMaxRun) { atomicOr(flag, kFlagLongRun); continue; }
         for (int a = 1; a < len; ++a) {
             const int32_t v = order[i + a];
             const int32_t e = end[v];
@@ -87,11 +101,25 @@ __global__ void k_key_cluster(int64_t n, const int32_t *order, const int32_t *ch
 // its chromosome plus, for every strand segment of the chromosome, the number of its junctions
 // that come before this one -- one binary search per segment (junctions are distinct, so the only
 // ties are across strands and break on the strand rank).
+// A chromosome or segment ends at the first key above its LAST possible key (all bits below the
+// field set), not at the first key of the next chromosome or strand: for chrom 2^25 - 1 that key
+// wraps to 0, and for strand 255 it carries into the chromosome field.  The segments then
+// partition [c_lo, c_hi), and the only one whose strand equals this junction's is its own, so every
+// rank lies in [c_lo, c_hi) whatever the keys hold.
+constexpr uint64_t kBelowChrom = (uint64_t(1) << 39) - 1, kBelowStrand = (uint64_t(1) << 31) - 1;
 __device__ __forceinline__ int64_t first_at_least(const uint64_t *key, int64_t lo, int64_t hi, uint64_t probe)
 {
     while (lo < hi) {
         const int64_t mid = (lo + hi) >> 1;
         if (key[mid] < probe) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+__device__ __forceinline__ int64_t first_above(const uint64_t *key, int64_t lo, int64_t hi, uint64_t last)
+{
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (key[mid] <= last) lo = mid + 1; else hi = mid;
     }
     return lo;
 }
@@ -106,11 +134,11 @@ __global__ void k_out_rank(int64_t n, const int32_t *order, const uint64_t *key_
         const int32_t j = order[i];
         const uint32_t my_end = (uint32_t)end[j];
         const int64_t c_lo = first_at_least(key_sorted, 0, i + 1, chrom << 39);
-        const int64_t c_hi = first_at_least(key_sorted, i + 1, n, (chrom + 1) << 39);
+        const int64_t c_hi = first_above(key_sorted, i + 1, n, (chrom << 39) | kBelowChrom);
         int64_t rank = c_lo;
         for (int64_t pos = c_lo; pos < c_hi;) {
             const uint32_t s2 = (uint32_t)(key_sorted[pos] >> 31) & 0xFFu;
-            const int64_t seg_end = first_at_least(key_sorted, pos + 1, c_hi, (chrom << 39) | ((uint64_t)(s2 + 1) << 31));
+            const int64_t seg_end = first_above(key_sorted, pos + 1, c_hi, key_sorted[pos] | kBelowStrand);
             if (s2 == strand) {
                 rank += i - pos;                                  // own segment: everything before this position
             } else {
@@ -373,7 +401,7 @@ int sd_cluster_build(int64_t n, const int32_t *chrom_rank, const int32_t *strand
     for (int attempt = 0; attempt < 2; ++attempt) {
         SD_CHECK_CUDA(cudaMemsetAsync(ws + w.misc, 0, 16, stream));
         if (attempt == 0) {
-            k_key_direct<<<g, kBlock, 0, stream>>>(n, chrom_rank, strand_rank, start, key_a, val_a);
+            k_key_direct<<<g, kBlock, 0, stream>>>(n, chrom_rank, strand_rank, start, end, key_a, val_a, d_flag);
             SD_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(cub_ws, cub_b, key_a, key_b, val_a, cluster_order, ni, 0, 64, stream));
             k_fix_ties<<<g, kBlock, 0, stream>>>(n, key_b, cluster_order, end, d_flag);
         } else {
@@ -402,14 +430,19 @@ int sd_cluster_build(int64_t n, const int32_t *chrom_rank, const int32_t *strand
         SD_CHECK_CUDA(cub::DeviceScan::ExclusiveSum(cub_ws, cub_b, (const int32_t *)deg_row, row_ptr, ni + 1, stream));
         if (int rc = check_launch("sd_cluster_build kernels")) return rc;
 
-        // the call's single synchronisation: long-run flag, 64-bit edge count (an overflowing prefix
-        // sum above only produces garbage that is never returned), nnz, component count
+        // the call's single synchronisation: flag word, 64-bit edge count (an overflowing prefix
+        // sum above only produces garbage that is never returned), nnz, component count.  Out-of-range
+        // input runs the whole build on aliased keys; every write stays inside the caller's arrays
+        // and the workspace (k_out_rank's ranks lie in [0, n)), and the call fails before any result.
         SD_CHECK_CUDA(cudaMemcpyAsync(&h_flag, d_flag, 4, cudaMemcpyDeviceToHost, stream));
         SD_CHECK_CUDA(cudaMemcpyAsync(&h_edges, d_edges, 8, cudaMemcpyDeviceToHost, stream));
         SD_CHECK_CUDA(cudaMemcpyAsync(&h_nnz, row_ptr + n, 4, cudaMemcpyDeviceToHost, stream));
         SD_CHECK_CUDA(cudaMemcpyAsync(&h_comp, comp_id + (n - 1), 4, cudaMemcpyDeviceToHost, stream));
         SD_CHECK_CUDA(cudaStreamSynchronize(stream));
-        if (!h_flag) break;
+        if (h_flag & kFlagBadInput)
+            return fail(SD_ERR_INVALID, "sd_cluster_build: a junction has chrom_rank outside [0, 2^25), strand_rank "
+                                        "outside [0, 256) or a negative start / end");
+        if (!(h_flag & kFlagLongRun)) break;
     }
     if (2 * h_edges > 0x7FFFFFFFull)
         return fail(SD_ERR_OVERFLOW, "sd_cluster_build: %llu adjacency entries do not fit int32 indices", 2 * h_edges);

@@ -339,6 +339,30 @@ int sd_signedrank_rows(int64_t n_events, int32_t n_samples, const void *ps, int6
                        int64_t row_begin, int64_t row_end,
                        int32_t *n_out, int64_t ld_n, double *stats_out, int64_t ld_stats, void *stream);
 
+/* ---- K9: Friedman test per event across conditions measured on the same subjects (compare_repeated) --
+ * For rows j in [row_begin, row_end) of ps (as K6): block (subject) b < n_blocks has one cell per
+ * condition c < n_conditions, ps[j, cols[c * n_blocks + b]] (a DEVICE int32 list, condition-major; no
+ * column listed twice), and
+ *   n_out[j]                         = n, the complete blocks (no NaN in any of their k cells)
+ *   mean_out[j * ld_mean + c]        = the mean of condition c over those blocks (float64 sum)
+ *   stats_out[j * ld_stats + 0, 1]   = Q, p
+ * with Q, p = scipy.stats.friedmanchisquare(*conditions, nan_policy='omit') (scipy 1.18.1) computed
+ * without its cancellation: cells ranked within their block with average ranks, D_c = 2 R_c - n (k + 1)
+ * and the tie term T exact integers, Q = 3 (k - 1) sum_c D_c^2 / (n (k^3 - k) - T) in one correctly
+ * rounded division, p = chi2.sf(Q, k - 1).  Every D_c == 0 gives Q == 0 and p == 1 exactly.  n == 0 (NaN
+ * means too), or every complete block tied throughout, gives Q = p = NaN (scipy gives NaN for the first,
+ * NaN or +inf for the second).  -0.0 ties +0.0; +-inf are ordinary values.  3 <= n_conditions <=
+ * SD_FRIEDMAN_MAX_CONDITIONS, n_blocks >= 1, n_blocks * n_conditions <= SD_RANKSUM_MAX_SAMPLES.  A column
+ * outside [0, n_samples) is never read: the rows get n = -1 and NaN means and statistics.  One
+ * asynchronous launch on `stream`, no synchronisation.
+ */
+#define SD_FRIEDMAN_MAX_CONDITIONS 256   /* chi2_sf handles df <= 255 */
+int sd_friedman_rows(int64_t n_events, int32_t n_samples, const void *ps, int64_t ld_ps, int dtype,
+                     int32_t n_conditions, int32_t n_blocks, const int32_t *cols,
+                     int64_t row_begin, int64_t row_end,
+                     int32_t *n_out, double *mean_out, int64_t ld_mean,
+                     double *stats_out, int64_t ld_stats, void *stream);
+
 /* ---- K4: intron-retention ratio ----------------------------------------------------
  * Replaces the arithmetic of ir_table.calculateIR (ir_table.py:118-132):
  *   ir[r,s] = median[r,s] / (median[r,s] + inc[r,s] + sum_{c in adj(r)} inc[c,s]),  x/0 -> NaN

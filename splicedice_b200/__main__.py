@@ -1,12 +1,14 @@
 """``python -m splicedice_b200 <command>``: the hot-path commands of the splicedice CLI
 (quant, counts_to_ps, pairwise, ir_table) with the reference's flags, compare_groups (a rank-sum
 test per event between two sample groups), compare_conditions (a Kruskal-Wallis test per event
-across any number of sample groups) and compare_paired (a signed-rank test per event between matched
-sample pairs), running on a B200.
+across any number of sample groups), compare_paired (a signed-rank test per event between matched
+sample pairs) and compare_repeated (a Friedman test per event across conditions measured on the same
+subjects), running on a B200.
 The remaining reference commands (BAM readers, the other downstream statistics) are out of scope."""
 import argparse
 
-from . import compare_conditions, compare_groups, compare_paired, counts_to_ps, ir_table, pairwise_fisher, quant
+from . import (compare_conditions, compare_groups, compare_paired, compare_repeated, counts_to_ps, ir_table,
+               pairwise_fisher, quant)
 
 COMMANDS = {
     "quant": quant,
@@ -16,6 +18,7 @@ COMMANDS = {
     "compare_groups": compare_groups,
     "compare_conditions": compare_conditions,
     "compare_paired": compare_paired,
+    "compare_repeated": compare_repeated,
 }
 
 

@@ -18,6 +18,7 @@ SD_QUANT_AUTO, SD_QUANT_GATHER, SD_QUANT_TILED = 0, 1, 2
 SD_QUANT_NARROW_TILES, SD_QUANT_VEC1, SD_QUANT_VEC2, SD_QUANT_GENERAL = 0x10000, 0x20000, 0x40000, 0x80000
 SD_RANKSUM_F32, SD_RANKSUM_F64 = 0, 1
 SD_RANKSUM_MAX_SAMPLES, SD_KRUSKAL_MAX_GROUPS, SD_SIGNEDRANK_MAX_PAIRS = 16384, 256, 8192
+SD_FRIEDMAN_MAX_CONDITIONS = 256
 ABI_VERSION = 1
 
 
@@ -77,6 +78,8 @@ _SIGNATURES = {
                                 c_int64, c_int64, _P, c_int64, _P, c_int64, _P, c_int64, _P]),
     "sd_signedrank_rows": (c_int, [c_int64, c_int32, _P, c_int64, c_int, c_int32, _P, _P,
                                    c_int64, c_int64, _P, c_int64, _P, c_int64, _P]),
+    "sd_friedman_rows": (c_int, [c_int64, c_int32, _P, c_int64, c_int, c_int32, c_int32, _P,
+                                 c_int64, c_int64, _P, _P, c_int64, _P, c_int64, _P]),
     "sd_bh_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int]),
     "sd_bh_adjust": (c_int, [c_int64, c_int64, _P, c_int64, _P, c_int64, c_int, _P, c_size_t, _P]),
     "sd_ir_ratio": (c_int, [c_int64, c_int32, _P, c_int64, _P, c_int64, _P, _P, _P, c_int64,

@@ -461,6 +461,61 @@ def signedrank_rows(ps, cols1, cols2, row_begin=0, row_end=None, out=None):
 
 
 # ---------------------------------------------------------------------------------------
+# K9
+# ---------------------------------------------------------------------------------------
+def friedman_rows(ps, blocks, row_begin=0, row_end=None, out=None):
+    """Friedman test per row across the conditions of a float32 / float64 CUDA PS matrix
+    (sd_friedman_rows; fully asynchronous): ``blocks`` is a host int array [n_blocks, k], row b the columns
+    of subject b under conditions 0 .. k - 1.  scipy.stats.friedmanchisquare(*conditions,
+    nan_policy='omit'): a block with a NaN cell is dropped, Q and p are NaN where no block is complete or
+    every complete block is tied throughout.  Returns a dict of CUDA views n (int32 [J]: complete blocks),
+    mean (float64 [J, k]: condition means over those blocks), Q and p (float64 [J]); only rows
+    [row_begin, row_end) are written.  ``out`` = (int32 [J], float64 [J, >= k], float64 [J, >= 2]) gives
+    the buffers behind those views.  The array is checked here: 2-D integer, 3 <= k <= 256, n_blocks >= 1,
+    n_blocks * k <= 16,384, every column in [0, S) and none listed twice."""
+    require_cuda()
+    if ps.dtype not in (torch.float32, torch.float64) or not ps.is_cuda or ps.dim() != 2:
+        raise TypeError("friedman_rows: ps must be a 2-D float32 / float64 CUDA tensor")
+    J, S = ps.shape
+    if J and S and ps.stride(1) != 1:
+        raise ValueError("friedman_rows: ps must be row-major")
+    h = np.asarray(blocks.cpu() if isinstance(blocks, torch.Tensor) else blocks)
+    if h.ndim != 2 or not np.issubdtype(h.dtype, np.integer):
+        raise ValueError("friedman_rows: blocks must be a 2-D integer array [n_blocks, k] of column indices")
+    nb, k = h.shape
+    if not 3 <= k <= native.SD_FRIEDMAN_MAX_CONDITIONS:
+        raise ValueError(f"friedman_rows: {k} conditions; 3 to {native.SD_FRIEDMAN_MAX_CONDITIONS} are supported")
+    if nb < 1:
+        raise ValueError("friedman_rows: no blocks")
+    if nb * k > native.SD_RANKSUM_MAX_SAMPLES:
+        raise ValueError(f"friedman_rows: {nb} blocks x {k} conditions = {nb * k} cells; "
+                         f"at most {native.SD_RANKSUM_MAX_SAMPLES}")
+    if h.min() < 0 or h.max() >= S:
+        raise ValueError(f"friedman_rows: a column outside [0, {S})")
+    if np.unique(h).size != h.size:
+        raise ValueError("friedman_rows: a column is listed twice")
+    dev = ps.device
+    # condition-major: the lanes of a warp hold consecutive subjects of one condition
+    d_cols = _i32(np.ascontiguousarray(h.T).reshape(-1), dev)
+    row_end = J if row_end is None else row_end
+    if out is None:
+        out = (torch.empty(J, dtype=torch.int32, device=dev), torch.empty((J, k), dtype=torch.float64, device=dev),
+               torch.empty((J, 2), dtype=torch.float64, device=dev))
+    n_out, mean, st = out
+    if (n_out.dtype != torch.int32 or mean.dtype != torch.float64 or st.dtype != torch.float64
+            or n_out.dim() != 1 or n_out.device != dev or n_out.shape[0] != J or (J and n_out.stride(0) != 1)
+            or any(t.dim() != 2 or t.device != dev or t.shape[0] != J or t.stride(1) != 1 for t in (mean, st))
+            or mean.shape[1] < k or st.shape[1] < 2):
+        raise TypeError("friedman_rows: out must be (int32 [J], float64 [J, >= k], float64 [J, >= 2]) on the PS device")
+    kind = native.SD_RANKSUM_F32 if ps.dtype == torch.float32 else native.SD_RANKSUM_F64
+    with torch.cuda.device(dev):
+        native.call("sd_friedman_rows", J, S, native.ptr(ps), ps.stride(0), kind, k, nb, native.ptr(d_cols),
+                    row_begin, row_end, native.ptr(n_out), native.ptr(mean), mean.stride(0), native.ptr(st),
+                    st.stride(0), _sp())
+    return dict(n=n_out, mean=mean[:, :k], Q=st[:, 0], p=st[:, 1])
+
+
+# ---------------------------------------------------------------------------------------
 # K4
 # ---------------------------------------------------------------------------------------
 def ir_ratio(median, counts, row_ptr=None, col_idx=None, row_begin=0, row_end=None):
